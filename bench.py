@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the batched Othello hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--games G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--games G] [--dump-outputs DIR]
 
 Workload (config.workload = "config3_random_playout"): G = 2**20 lock-step random-playout games
 PER GPU from the standard opening, every position and move written to HBM (SoA trajectory).  A
@@ -22,6 +22,11 @@ step).  Games are independent, so N GPUs run N shards with no data-path collecti
               kind of games on all host cores for a bounded time (N=1, rank 0 only)
 
 `--impl reference` times only that CPU path and prints the same JSON shape.
+
+`--dump-outputs DIR` writes what the last timed launch returned (nplies, final positions and trajectories of a fixed
+sample of its games, see sample_outputs) and the batch totals of all timed steps, from which `value` is computed, as
+DIR/<name>.npy.  The games of a step depend only on --games, --warmup and
+--steps, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -447,6 +452,46 @@ def config5_table_extra(dev, G=1 << 16, iters=3, warm=1, random_plies=10):
                     "bit-identical to the reference loop) -> four fits on sampled table entries"}
 
 
+DUMP_GAMES = 1 << 18          # --dump-outputs: games of the last timed step whose per-game results are written
+DUMP_TRAJ_GAMES = 1 << 12     # ... and how many of them also have their whole trajectory written (28 MB in all)
+
+
+def _bits_halves(a):
+    """int64 bit patterns -> float64 [..., 2] (low, high 32-bit halves): exact, where one float64 would round"""
+    import numpy as np
+    u = a.view(np.uint64)
+    return np.stack([u & 0xFFFFFFFF, u >> 32], axis=-1).astype(np.float64)
+
+
+def sample_outputs(po, gid0, totals):
+    """What the caller of one ops.playout launch receives, on a fixed seeded sample of its games (game ids from gid0):
+    nplies and final positions of DUMP_GAMES games, trajectories of DUMP_TRAJ_GAMES of them.  Bitboards are (low, high)
+    halves; trajectory entries past a game's end, which the kernel leaves unspecified, are -1.  ``totals`` (int64 [4]:
+    plies, sum of n_black - n_white, Black wins, White wins) is written as it stands."""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(0)
+    T = po.t_max
+    idx = np.sort(rng.choice(po.n_games, size=min(po.n_games, DUMP_GAMES), replace=False))
+    tix = np.sort(rng.choice(idx, size=min(idx.size, DUMP_TRAJ_GAMES), replace=False))
+    nplies = po.nplies.cpu().numpy()
+    sel = torch.from_numpy(tix).to(po.nplies.device)
+    tb = _bits_halves(po.black.index_select(1, sel).cpu().numpy())           # [T+1][n][2]
+    tw = _bits_halves(po.white.index_select(1, sel).cpu().numpy())
+    tm = po.move.index_select(1, sel).cpu().numpy().astype(np.float32)       # [T][n]
+    t = np.arange(T + 1)[:, None]
+    end = np.minimum(nplies[tix], T)[None, :]
+    tb[t > end] = -1
+    tw[t > end] = -1
+    tm[t[:-1] >= end] = -1
+    return {"game_id": (gid0 + idx).astype(np.float64), "nplies": nplies[idx].astype(np.float32),
+            "final_black": _bits_halves(po.final_black.cpu().numpy()[idx]),
+            "final_white": _bits_halves(po.final_white.cpu().numpy()[idx]),
+            "trajectory_game_id": (gid0 + tix).astype(np.float64),
+            "trajectory_black": tb, "trajectory_white": tw, "trajectory_move": tm,
+            "totals": totals.cpu().numpy().astype(np.float64)}
+
+
 def run_b200_arm(args):
     import ctypes
     import torch
@@ -519,6 +564,11 @@ def run_b200_arm(args):
     ev_end.record(cur)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    # taken now: the launches timed alone below reuse the buffers of the timed steps.  The totals, from which `value`
+    # is computed, are those of all K timed steps (each stream accumulates its own).
+    i_last = W + K - 1
+    outputs = (sample_outputs(pos[i_last % 2], gid_base + i_last * G, tot[0] + tot[1])
+               if args.dump_outputs and rank == 0 else None)
     # time a launch spends in its stream (launches of the two streams overlap, so these add up to more than the total)
     step_ms = [(ev_start if i < 2 else evs[i - 2]).elapsed_time(evs[i]) for i in range(K)]
     total_ms = ev_start.elapsed_time(ev_end)
@@ -752,6 +802,11 @@ def run_b200_arm(args):
             cb["config1_single_game_facade"] = config1_facade()
             line["cpu_baseline"] = cb
         print(json.dumps(line))
+    if outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -770,7 +825,13 @@ def main():
                          "90 / (steps + warmup) clamped to [2, 20] per step of --impl reference)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 4 / config 5 objects")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (a fixed sample of its games, rank "
+                         "0's with several GPUs) and the totals of all of them as DIR/<name>.npy in float32 / float64, "
+                         "for comparing two builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3                      # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

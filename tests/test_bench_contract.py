@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -57,3 +58,49 @@ def test_b200_arm_line():
     assert c5t["iteration_ms"] > 0 and c5t["table_keys"] > 0 and len(c5t["parameters"]) == 36
     assert d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] > 0
     assert d["clocks"]["sm_mhz"] is None or d["clocks"]["sm_mhz"] > 500
+
+
+def _u64(halves):
+    return halves[..., 0].astype(np.uint64) | (halves[..., 1].astype(np.uint64) << np.uint64(32))
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_games_of_the_last_timed_step(tmp_path, oracle):
+    G, K, W = 8192, 2, 3
+    args = ["--steps", str(K), "--warmup", str(W), "--games", str(G), "--no-cpu-baseline", "--no-extra", "--dump-outputs"]
+    d = run(args + [str(tmp_path / "a")], timeout=600)
+    assert d["steps"] == K and d["gpu_launches"] == K
+    run(args + [str(tmp_path / "b")], timeout=600)
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(p.name for p in (tmp_path / "b").iterdir())
+    out, total = {}, 0
+    for n in names:
+        a = np.load(tmp_path / "a" / n)
+        assert a.dtype in (np.float32, np.float64)
+        assert np.array_equal(a, np.load(tmp_path / "b" / n))              # same arguments, same outputs
+        out[n[:-4]] = a
+        total += a.nbytes
+    assert total <= 64 << 20
+    # step i plays games i*G .. i*G+G-1 of seed 1; the last timed step is i = W+K-1
+    gid0 = (W + K - 1) * G
+    ref = oracle.playout(1, gid0, G)
+    g = out["game_id"].astype(np.int64) - gid0
+    assert g.size == G and np.array_equal(g, np.arange(G))
+    assert np.array_equal(out["nplies"], ref["nplies"])
+    assert np.array_equal(_u64(out["final_black"]), ref["final_black"])
+    assert np.array_equal(_u64(out["final_white"]), ref["final_white"])
+    tg = out["trajectory_game_id"].astype(np.int64) - gid0
+    t = np.arange(ref["black"].shape[0])[:, None]
+    pos_ok = t <= ref["nplies"][tg][None, :]
+    assert np.array_equal(out["trajectory_black"][..., 0] >= 0, pos_ok)
+    assert np.array_equal(_u64(out["trajectory_black"])[pos_ok], ref["black"][:, tg][pos_ok])
+    assert np.array_equal(_u64(out["trajectory_white"])[pos_ok], ref["white"][:, tg][pos_ok])
+    mv_ok = t[:-1] < ref["nplies"][tg][None, :]
+    assert np.array_equal(out["trajectory_move"] >= 0, mv_ok)
+    assert np.array_equal(out["trajectory_move"][mv_ok], ref["move"][:, tg][mv_ok])
+    # the totals `value` is computed from: plies, disc difference and wins over the games of all K timed steps
+    allg = oracle.playout(1, W * G, K * G, trajectory=False)
+    nb, nw = np.bitwise_count(allg["final_black"]).astype(np.int64), np.bitwise_count(allg["final_white"]).astype(np.int64)
+    want = [allg["nplies"].sum(dtype=np.int64), (nb - nw).sum(), (nb > nw).sum(), (nw > nb).sum()]
+    assert out["totals"].tolist() == [float(v) for v in want]
+    assert d["value"] == pytest.approx(want[0] / (d["ms_per_step"] * K * 1e-3), rel=1e-9)

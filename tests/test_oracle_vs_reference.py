@@ -1,7 +1,7 @@
-"""Live differential check: oracle vs the reference's own board.py on fresh random positions.
-
-Runs only where the reference is reachable (/root/reference in the build container, or
-oracle/_ref on a box that received it); elsewhere the golden vectors are the pin.
+"""The oracle against the reference.  The two game tests play fresh games on the reference's own board.py and run
+only where its sources are reachable (oracle/_ref, see oracle/build_ref.py); without them the stored reference games
+of tests/test_oracle_golden.py are the pin.  The evaluation test uses the reference's counts() stored with the golden
+games and runs everywhere.
 """
 import numpy as np
 import pytest
@@ -9,9 +9,11 @@ import pytest
 from oracle import refshim
 from oracle import make_golden as mg
 
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference not present on this box")
+live = pytest.mark.skipif(not refshim.available(), reason="needs the original project's sources (oracle/_ref, see "
+                          "oracle/build_ref.py), which are not part of the repository")
 
 
+@live
 def test_random_games_against_live_reference(oracle):
     ns = refshim.load()
     rows = ns.ppml.ProgressPositionMovesParameter().default_value()
@@ -28,6 +30,7 @@ def test_random_games_against_live_reference(oracle):
         assert r['move'][:len(g['plies']), 0].tolist() == [p['move'] for p in g['plies']]
 
 
+@live
 def test_greedy_games_against_live_reference(oracle):
     ns = refshim.load()
     rows = ns.ppml.ProgressPositionMovesParameter().default_value()
@@ -38,21 +41,24 @@ def test_greedy_games_against_live_reference(oracle):
         assert int(r['nplies'][0]) == len(g['plies'])
 
 
-def test_eval_against_counts_dot(oracle):
-    ns = refshim.load()
-    rb = ns.board
+def test_eval_against_counts_dot(oracle, golden_games):
+    """the oracle's linear form against the dot product of the reference's own counts() of every position of the
+    golden games that carry them (recorded by oracle/make_golden.py as feat_O / feat_X)"""
     rng = np.random.RandomState(3)
     w = np.concatenate([rng.uniform(-2, 2, size=(4, 9)), rng.uniform(-1, 1, size=(4, 1))], axis=1)
-    r = oracle.playout(13, 0, 4)
-    for g in range(4):
-        for t in range(0, int(r['nplies'][g]) + 1, 7):
-            bb, ww = int(r['black'][t, g]), int(r['white'][t, g])
-            B = rb.Board()
-            for s in range(64):
-                B.set(rb.Black if (bb >> s) & 1 else rb.White if (ww >> s) & 1 else rb.Empty, s & 7, s >> 3)
-            for side, colour in (('O', 1), ('X', 2)):
-                f = ns.ppml.counts(mg.book_of(B), side)
+    checked = 0
+    for g in golden_games:
+        pos = g['positions']
+        if 'feat_O' not in pos[0]:
+            continue
+        b = np.array([int(p['b'], 16) for p in pos], dtype=np.uint64)
+        ww = np.array([int(p['w'], 16) for p in pos], dtype=np.uint64)
+        for key, colour in (('feat_O', 1), ('feat_X', 2)):
+            got = oracle.evaluate(b, ww, colour, w)
+            for p, v in zip(pos, got):
+                f = p[key]
                 row = 0 if f[0] <= 16 else 1 if f[0] <= 32 else 2 if f[0] <= 48 else 3
                 want = float(np.dot(w[row, :9], np.array(f[1:], dtype=np.float64)) + w[row, 9])
-                got = float(oracle.evaluate([bb], [ww], colour, w)[0])
-                assert abs(got - want) <= 1e-12 * max(1.0, abs(want))
+                assert abs(float(v) - want) <= 1e-12 * max(1.0, abs(want))
+                checked += 1
+    assert checked >= 900
