@@ -15,7 +15,8 @@
  *     string that does not parse (put_s returns -1);
  *   - "_host" functions take HOST pointers and run on the context's own stream and workspace;
  *     all others take DEVICE pointers, launch asynchronously on `stream` (a cudaStream_t passed
- *     as void*), allocate nothing and keep no global state;
+ *     as void*), allocate nothing and keep no global state -- except othello_playout with the
+ *     random engine, which keeps its opening book on the device (see there);
  *   - every function returns 0 on success, a positive cudaError_t value, or a negative
  *     OTHELLO_E_* code.  othello_error_string() explains both.
  */
@@ -143,6 +144,11 @@ typedef struct {
     uint16_t *summary;
 } othello_playout_args;
 
+/* Device memory kept by the library: the random engine takes the first 8 plies of games that start from the
+ * standard opening with Black to move from an opening book (the game tree of those plies, 455 221 nodes).  The
+ * first random-engine call on a device allocates 14.6 MB there, uploads the book synchronously (the host keeps its
+ * 14.6 MB copy) and keeps it until the process exits.  A call on a stream that is being captured into a CUDA graph
+ * does not upload it: its kernel plays those plies itself.  Results do not depend on either. */
 int othello_playout(const othello_playout_args *args, void *stream);
 
 /* ---- perft ---------------------------------------------------------------------------------- */

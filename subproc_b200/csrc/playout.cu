@@ -1,21 +1,31 @@
 // playout.cu -- GameRunner.play_a_game (game_runner.py:165-201) for millions of games at once.
 //
 // One thread owns one game from the first ply to the last: the position lives in four 32-bit
-// registers (own/opp bitboards), a ply is ~385 integer instructions (fastboard.cuh) and touches memory
+// registers (own/opp bitboards), a ply is ~300 integer instructions (fastboard.cuh) and touches memory
 // only to append the position and the move to the SoA trajectory [t][game] (a warp writes
 // 32 consecutive u64 = 256 B per array per ply).  The warp runs in lock step; games that end
-// early idle until the longest game of the warp is over.  Nothing is read from HBM after the
-// start position.
+// early idle until the longest game of the warp is over.  A warp whose games all start from the
+// standard opening with Black to move takes its first OB_PLAYOUT_BOOK_DEPTH plies from the opening
+// book (opening_book.cuh): per ply the loads of one 32-byte node of a 14.6 MB table; after that
+// nothing is read from memory.
 //
 // The loop is the reference's: positions are recorded before every ply and once at the end
 // (recorder.add, game_runner.py:170,159); the side to move asks go_for (game_runner.py:133-152),
 // which may substitute a uniformly random move for the engine's, an engine with no move answers
 // 'ps' and the pass is a ply of its own (board.py:194-195,203-208); the game stops when neither
 // colour can move (board.py:57-58).
+#include <atomic>
+#include <cstdio>
+#include <cstdlib>
+#include <mutex>
+#include <vector>
 #include "playout_common.cuh"
+#include "opening_book.cuh"
 
 using namespace ob;
 using namespace obp;
+using obb::BookNode;
+using obb::kBookDepth;
 
 namespace {
 
@@ -83,13 +93,46 @@ __device__ __forceinline__ bool play_ply(Game &g, bool black_moves, u32 key, int
     return true;
 }
 
+// The first kBookDepth plies of a game from the standard opening with Black to move, walked down the opening book
+// instead of played: the same draw as play_ply picks the same move (the k-th child is the k-th legal move), and the
+// same rows are written.  No ply of the book is a pass, so the game goes on with Black to move (kBookDepth is even).
+template <int TRAJ>
+__device__ __forceinline__ void play_book(Game &g, u32 key, int t_max, int64_t stride, const BookNode *__restrict__ book,
+                                          u64 *__restrict__ traj_black, u64 *__restrict__ traj_white,
+                                          uint8_t *__restrict__ traj_move)
+{
+    const uint4 *node = reinterpret_cast<const uint4 *>(book);       // two 16-byte halves per node: position, links
+    uint4 links = __ldg(node + 1);
+    u64 black = OTHELLO_START_BLACK, white = OTHELLO_START_WHITE;
+#pragma unroll
+    for (int t = 0; t < kBookDepth; t++) {
+        if (TRAJ == 2 || (TRAJ == 1 && t <= t_max)) {
+            __stcs(traj_black + g.off, black);
+            __stcs(traj_white + g.off, white);
+        }
+        const u32 r = rng_draw_fma(key, (u32)t, 1u, obf::kOpaqueOne);
+        const u32 child = links.x + rng_below(r, links.y & 0xffu);
+        links = __ldg(node + 2 * child + 1);
+        const uint4 pos = __ldg(node + 2 * child);                   // (TRAJ == 0: only the last one is kept)
+        black = obf::pack(pos.x, pos.y);
+        white = obf::pack(pos.z, pos.w);
+        if (TRAJ == 2 || (TRAJ == 1 && t < t_max)) __stcs(traj_move + g.off, (uint8_t)(links.y >> 8));
+        if (TRAJ) g.off += (unsigned)stride;
+    }
+    g.own = black;
+    g.opp = white;
+    g.t = kBookDepth;
+}
+
 // UNIFORM: no per-game turn0 -- every game starts with Black, so the loop is unrolled over the two colours
 template <int TRAJ, bool UNIFORM>
 // (128 threads x >= 10 CTAs per SM measured best on B200: 64/128/256 threads and 9..12 CTAs are within 2 %)
 #if !defined(OB_PLAYOUT_CTAS)
 #define OB_PLAYOUT_CTAS 10
 #endif
-__global__ void __launch_bounds__(kThreads, OB_PLAYOUT_CTAS) playout_kernel(const othello_playout_args a)
+// book: the opening book on this device, or nullptr
+__global__ void __launch_bounds__(kThreads, OB_PLAYOUT_CTAS) playout_kernel(const othello_playout_args a,
+                                                                            const BookNode *__restrict__ book)
 {
     __shared__ __align__(16) u64 ray_s[obf::kRayTable64];
     ob::fill_tables<kThreads>(ray_s);
@@ -97,11 +140,15 @@ __global__ void __launch_bounds__(kThreads, OB_PLAYOUT_CTAS) playout_kernel(cons
     const Rays rays = {ray_s};
     const int64_t gi = (int64_t)blockIdx.x * kThreads + threadIdx.x;
     const bool live = gi < a.n_games;                  // lanes past the batch only take part in the totals
+    const u64 b0 = live && a.black0 ? a.black0[gi] : OTHELLO_START_BLACK;
+    const u64 w0 = live && a.white0 ? a.white0[gi] : OTHELLO_START_WHITE;
+    bool black_moves = UNIFORM || !live ? true : (a.turn0[gi] == OTHELLO_BLACK);
+    // the whole warp takes the book or none of it (lanes past the batch do not object)
+    bool booked = book != nullptr;
+    if (booked && (a.black0 || !UNIFORM))
+        booked = __all_sync(0xffffffffu, b0 == OTHELLO_START_BLACK && w0 == OTHELLO_START_WHITE && black_moves);
     int plies = 0, n_black = 0, n_white = 0;
     if (live) {
-        const u64 b0 = a.black0 ? a.black0[gi] : OTHELLO_START_BLACK;
-        const u64 w0 = a.white0 ? a.white0[gi] : OTHELLO_START_WHITE;
-        bool black_moves = UNIFORM ? true : (a.turn0[gi] == OTHELLO_BLACK);
         Game g;
         g.own = black_moves ? b0 : w0; g.opp = black_moves ? w0 : b0;
         g.t = 0;
@@ -110,6 +157,7 @@ __global__ void __launch_bounds__(kThreads, OB_PLAYOUT_CTAS) playout_kernel(cons
         const u32 key = rng_key(a.seed, a.gid0 + (u64)gi);
         const int t_max = a.t_max;
         const int64_t stride = a.stride;
+        if (booked) play_book<TRAJ>(g, key, t_max, stride, book, (u64 *)a.traj_black, (u64 *)a.traj_white, a.traj_move);
 
         if (UNIFORM) {
             for (;;) {
@@ -130,22 +178,67 @@ __global__ void __launch_bounds__(kThreads, OB_PLAYOUT_CTAS) playout_kernel(cons
     add_totals(a.totals, live, plies, n_black, n_white);
 }
 
+// The opening book on the current device in *book: the tree is built on the host once per process and uploaded once
+// per device, by the first launch that can use it, and kept until the process exits.  The upload is complete before
+// any kernel is queued, so launches on every stream see the whole table.  *book stays nullptr while `s` is being
+// captured into a graph, whose capture an upload would break: the kernel then plays those plies itself, with the same
+// results.
+int book_on_device(cudaStream_t s, const BookNode **book)
+{
+    *book = nullptr;
+    cudaStreamCaptureStatus capture;
+    OB_CUDA(cudaStreamIsCapturing(s, &capture));
+    if (capture != cudaStreamCaptureStatusNone) return 0;
+    constexpr int kMaxDevices = 64;
+    static std::atomic<const BookNode *> on_device[kMaxDevices];
+    static std::mutex upload;
+    static std::vector<BookNode> tree;
+    int dev;
+    OB_CUDA(cudaGetDevice(&dev));
+    if (dev >= kMaxDevices) return 0;
+    if ((*book = on_device[dev].load(std::memory_order_acquire)) != nullptr) return 0;
+    std::lock_guard<std::mutex> lock(upload);
+    if ((*book = on_device[dev].load(std::memory_order_relaxed)) != nullptr) return 0;
+    if (tree.empty() && !obb::build_book(kBookDepth, tree)) {
+        fprintf(stderr, "othello_b200: a position of the opening book has no legal move\n");
+        abort();
+    }
+    const size_t bytes = tree.size() * sizeof(BookNode);
+    BookNode *d = nullptr;
+    cudaStream_t copy = nullptr;
+    cudaError_t e = cudaMalloc((void **)&d, bytes);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&copy, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d, tree.data(), bytes, cudaMemcpyHostToDevice, copy);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(copy);
+    if (copy) cudaStreamDestroy(copy);
+    if (e != cudaSuccess) {
+        cudaFree(d);
+        return (int)e;
+    }
+    on_device[dev].store(d, std::memory_order_release);
+    *book = d;
+    return 0;
+}
+
 int launch(const othello_playout_args &a, cudaStream_t s)
 {
     const unsigned blocks = ob_blocks(a.n_games, kThreads);
+    if (a.traj_black && (int64_t)(a.t_max + 2) * a.stride >= (1ll << 32)) return OTHELLO_E_INVALID;   // 32-bit trajectory index
+    const BookNode *book = nullptr;                                          // (OB_PLAYOUT_BOOK_DEPTH=0: no book)
+    if (kBookDepth > 0)
+        if (const int rc = book_on_device(s, &book)) return rc;
     if (a.traj_black) {
-        if ((int64_t)(a.t_max + 2) * a.stride >= (1ll << 32)) return OTHELLO_E_INVALID;   // 32-bit trajectory index
         const bool fits = a.black0 == nullptr && a.t_max >= 120;             // every game from the standard opening fits
         if (a.turn0) {
-            if (fits) playout_kernel<2, false><<<blocks, kThreads, 0, s>>>(a);
-            else playout_kernel<1, false><<<blocks, kThreads, 0, s>>>(a);
+            if (fits) playout_kernel<2, false><<<blocks, kThreads, 0, s>>>(a, book);
+            else playout_kernel<1, false><<<blocks, kThreads, 0, s>>>(a, book);
         } else {
-            if (fits) playout_kernel<2, true><<<blocks, kThreads, 0, s>>>(a);
-            else playout_kernel<1, true><<<blocks, kThreads, 0, s>>>(a);
+            if (fits) playout_kernel<2, true><<<blocks, kThreads, 0, s>>>(a, book);
+            else playout_kernel<1, true><<<blocks, kThreads, 0, s>>>(a, book);
         }
     } else {
-        if (a.turn0) playout_kernel<0, false><<<blocks, kThreads, 0, s>>>(a);
-        else playout_kernel<0, true><<<blocks, kThreads, 0, s>>>(a);
+        if (a.turn0) playout_kernel<0, false><<<blocks, kThreads, 0, s>>>(a, book);
+        else playout_kernel<0, true><<<blocks, kThreads, 0, s>>>(a, book);
     }
     return ob_launch_status();
 }
