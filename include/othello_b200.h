@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define OTHELLO_ABI_VERSION 3
+#define OTHELLO_ABI_VERSION 4
 
 #define OTHELLO_EMPTY 0
 #define OTHELLO_BLACK 1
@@ -168,6 +168,31 @@ int othello_perft(uint64_t black, uint64_t white, int turn, int depth, void *wor
                   uint64_t *result, void *stream);
 int othello_perft_async(uint64_t black, uint64_t white, int turn, int depth, int part, int nparts,
                         void *workspace, int64_t workspace_bytes, uint64_t *result, void *stream);
+
+/* ---- exact endgame solver ------------------------------------------------------------------- */
+
+/* The perfect-play value and best move of n positions, one lane per position (negamax, alpha-beta).
+ *   value: own - opponent discs of the terminal position reached when both sides play perfectly, "own" = the side
+ *          to move; the game ends when neither side can move (Board.is_game_over, board.py:57-58) and a pass is a
+ *          ply.  Empty squares left at the end are NOT given to the winner: this is the reference's own scoring
+ *          (winner by disc count, game_runner.py:194-199; learner target own - opp final discs,
+ *          progress_position_moves_learn.py:55), not the Edax / WTHOR convention.  Range -64..64.
+ *   move:  the lowest square (x + 8*y) among the moves that reach the value; OTHELLO_PASS when the side to move has
+ *          no move but the game is not over (value = minus the value with the other side to move);
+ *          OTHELLO_NO_MOVE when the game is over (value = the disc difference).
+ *   A position with more than OTHELLO_SOLVE_MAX_EMPTIES empty squares, or with black & white != 0, gets value
+ *   OTHELLO_SOLVE_REFUSED and move OTHELLO_NO_MOVE; the rest of the batch is solved normally.
+ *   nodes: positions the search visited, per position (benchmarking only): a function of the position alone,
+ *          whatever the batch around it.  May be NULL.
+ * turn: [n] side to move (OTHELLO_BLACK, anything else = White), or NULL = Black.  Asynchronous on `stream`,
+ * DEVICE pointers.  workspace: DEVICE scratch, >= othello_solve_workspace_bytes(); holds the work counter of the
+ * persistent grid, which the call resets itself.  n = 0 is a no-op. */
+#define OTHELLO_SOLVE_MAX_EMPTIES 24
+#define OTHELLO_SOLVE_REFUSED   (-128)
+#define OTHELLO_NO_MOVE          255
+int64_t othello_solve_workspace_bytes(void);
+int othello_solve(const uint64_t *black, const uint64_t *white, const uint8_t *turn, int32_t *value, uint8_t *move,
+                  uint64_t *nodes, int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
 
 /* ---- learner sufficient statistics ---------------------------------------------------------- */
 

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libothello_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 u64p = ctypes.POINTER(ctypes.c_uint64)
 u8p = ctypes.POINTER(ctypes.c_uint8)
@@ -64,6 +64,8 @@ SIGNATURES = {
                                      u64p, vp]),
     "othello_perft_async": (ctypes.c_int, [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                            ctypes.c_int, vp, i64, vp, vp]),
+    "othello_solve_workspace_bytes": (i64, []),
+    "othello_solve": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, i64, vp, i64, vp]),
     "othello_learn_accumulate": (ctypes.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, vp, vp, vp]),
     "othello_learn_stats": (ctypes.c_int, [vp, vp, vp]),
     "othello_learn_refit": (ctypes.c_int, [vp, i32, vp, vp, vp, vp, vp, vp]),

@@ -3,7 +3,7 @@
 The reference plays a game by spawning two engines with ``subprocess.Popen(path, shell=True)`` and
 talking to them over pipes (game_runner.py:11-102).  This module is such an engine:
 
-    python -m subproc_b200.edax_engine [--policy random|greedy] [--param FILE] [--name NAME] [--seed S]
+    python -m subproc_b200.edax_engine [--policy random|greedy] [--param FILE] [--name NAME] [--seed S] [--exact N]
     python -m subproc_b200.edax_engine -h "<64 chars> <turn char>"      # feature dump
 
 Protocol, as read by the reference's regexes:
@@ -17,6 +17,9 @@ Protocol, as read by the reference's regexes:
 the turn character -- what parameter_learn_from_edax_protocol.counts parses (:7-13).  Which colour
 the external engines meant is not pinned by the reference (the engines are not vendored).
 
+``--exact N`` (default 0 = off): with at most N empty squares left, ``go`` plays the perfect-play move of the exact
+endgame solver (ops.solve; the lowest square among the best moves) instead of the policy's.  N <= 24.
+
 Move choice and all rules run through the CUDA kernels (subproc_b200.board / ops).
 """
 import argparse
@@ -26,10 +29,15 @@ import sys
 class Backend(object):
     """rules + policy on the GPU"""
 
-    def __init__(self, policy='random', weights=None, seed=0, device=None):
+    def __init__(self, policy='random', weights=None, seed=0, device=None, exact_empties=0):
         from . import board
+        if exact_empties:
+            from . import ops
+            if not 0 < exact_empties <= ops.SOLVE_MAX_EMPTIES:
+                raise ValueError("exact_empties must be in 0..%d" % ops.SOLVE_MAX_EMPTIES)
         self.board_mod = board
         self.policy = policy
+        self.exact_empties = exact_empties
         self.weights = weights
         self.seed = seed
         self.device = device
@@ -50,12 +58,17 @@ class Backend(object):
         legal = self.b.puttables(self.b.turn)
         if not legal:
             return 'PS'
+        own, opp = self.b._pair(self.b.turn)
+        if 64 - bin(own | opp).count("1") <= self.exact_empties:
+            dev = torch.device("cuda", self.b._ctx_index())
+            _, move, _ = ops.solve(ops.bits_tensor([own], dev), ops.bits_tensor([opp], dev))
+            s = int(move[0])
+            return self.b.handstr_from_coord(s & 7, s >> 3).upper()
         if self.policy == 'random' or len(legal) == 1:
             key = (self.seed * 1000003 + self.games * 7919 + int(self.b.nturn)) & 0xFFFFFFFF
             x, y = legal[key % len(legal)] if self.policy == 'random' else legal[0]
             return self.b.handstr_from_coord(x, y).upper()
         dev = torch.device("cuda", self.b._ctx_index())
-        own, opp = self.b._pair(self.b.turn)
         n = len(legal)
         sq = torch.tensor([x + 8 * y for x, y in legal], dtype=torch.uint8, device=dev)
         o = ops.bits_tensor([own] * n, dev)
@@ -137,11 +150,12 @@ def main(argv=None):
     ap.add_argument("--param", default=None, help="38-byte parameter file (paramgen format)")
     ap.add_argument("--name", default="b200")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--exact", type=int, default=0, help="play perfectly with at most this many empties (0 = off)")
     args = ap.parse_args(argv)
     from . import parameter, paramgen
     P = parameter.ProgressPositionMovesParameter()
     weights = P.weights_table(paramgen.read_data(args.param) if args.param else None)
-    EdaxFrontEnd(Backend(args.policy, weights, args.seed), args.name).serve()
+    EdaxFrontEnd(Backend(args.policy, weights, args.seed, exact_empties=args.exact), args.name).serve()
     return 0
 
 

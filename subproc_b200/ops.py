@@ -303,6 +303,40 @@ def perft_distributed(depth, black=START_BLACK, white=START_WHITE, turn=BLACK, d
     return nodes
 
 
+NO_MOVE = 255                                    # OTHELLO_NO_MOVE: the game is over (or the position was refused)
+SOLVE_MAX_EMPTIES = 24                           # OTHELLO_SOLVE_MAX_EMPTIES
+SOLVE_REFUSED = -128                             # OTHELLO_SOLVE_REFUSED
+_solve_ws = {}                                   # (device, stream) -> workspace: the work counter of one call at a time
+
+
+def solve(black, white, turn=None, nodes=False):
+    """Exact endgame values (othello_solve): (value int32 [n], move uint8 [n], nodes int64 [n] or None).
+
+    value = own - opponent discs at the end of perfect play, own = the side to move (``turn``: uint8 [n], 1 = Black,
+    None = Black to move everywhere); empty squares left at the end are not given to the winner.  move = the lowest
+    square reaching the value, PASS when the mover must pass, NO_MOVE when the game is over.  Positions with more
+    than SOLVE_MAX_EMPTIES empties or overlapping colours get SOLVE_REFUSED / NO_MOVE.  ``nodes``: also return the
+    positions the search visited, per position (benchmarking)."""
+    n = black.numel()
+    dev = black.device
+    value = torch.empty(n, dtype=torch.int32, device=dev)
+    move = torch.empty(n, dtype=torch.uint8, device=dev)
+    cnt = torch.empty(n, dtype=torch.int64, device=dev) if nodes else None
+    nbytes = int(_lib.lib().othello_solve_workspace_bytes())
+    with torch.cuda.device(dev):
+        stream = _stream(black)
+        # calls on one stream run one after the other; calls on different streams may overlap, so each stream has
+        # its own counter
+        ws = _solve_ws.get((dev, stream.value))
+        if ws is None:
+            ws = _solve_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        _lib.check(_lib.lib().othello_solve(
+            _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
+            _req(value, torch.int32, n, "value"), _req(move, torch.uint8, n, "move"), _opt(cnt, torch.int64, n, "nodes"),
+            n, _req(ws, torch.uint8, nbytes, "workspace"), nbytes, stream), "othello_solve")
+    return value, move, cnt
+
+
 def decay_table(t_max, lam=0.90):
     """decay[k] = lam ** k in fp64, evaluated by CPython exactly like `self.l ** turn_left`
     (progress_position_moves_learn.py:24,55)."""
