@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define OTHELLO_ABI_VERSION 4
+#define OTHELLO_ABI_VERSION 5
 
 #define OTHELLO_EMPTY 0
 #define OTHELLO_BLACK 1
@@ -193,6 +193,38 @@ int othello_perft_async(uint64_t black, uint64_t white, int turn, int depth, int
 int64_t othello_solve_workspace_bytes(void);
 int othello_solve(const uint64_t *black, const uint64_t *white, const uint8_t *turn, int32_t *value, uint8_t *move,
                   uint64_t *nodes, int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
+
+/* ---- midgame search ------------------------------------------------------------------------- */
+
+/* The depth-limited minimax value and best move of n positions on the linear evaluation, one lane per position
+ * (negamax, alpha-beta).
+ *   score: every node of the tree is scored from the ROOT mover's side, score(P, O) = W[phase(P|O)] . (mobility(P),
+ *          a..h of P) + W[phase][9], P = the root mover's discs: exactly the fp32 value othello_eval(..., side = the
+ *          root mover, weights) returns, and the one the greedy policy computes for a successor.
+ *   tree:  plies alternate from the root; a ply is a legal move, or a pass when the side to move has no move but the
+ *          other side has one.  A pass is a ply and uses one level of depth (as in board.py, perft and the playout
+ *          kernels).  A node is a leaf `depth` plies below the root, or when neither side can move; every leaf,
+ *          game-over leaves included, is scored with score().
+ *   value: plain minimax over the fp32 leaf scores, max on the root mover's plies, min on the opponent's.  max and
+ *          min are exact, so the value does not depend on move order, pruning or scheduling.  -0.0 is returned as
+ *          +0.0.
+ *   move:  the lowest square (x + 8*y) whose subtree reaches the value; OTHELLO_PASS when the root mover must pass
+ *          (value: the passed position searched to depth - 1); OTHELLO_NO_MOVE when the game is over (value:
+ *          score(root)).  depth = 1 is the greedy policy (OTHELLO_POLICY_GREEDY) exactly: the same move on every
+ *          position, the value the evaluation of that successor.
+ *   A position with black & white != 0 gets value NaN and move OTHELLO_NO_MOVE; the rest of the batch is searched.
+ *   nodes: positions the search visited, per position (benchmarking only): a function of (position, depth, weights)
+ *          alone, whatever the batch around it.  May be NULL.
+ * weights: DEVICE float [OTHELLO_PHASES][OTHELLO_WEIGHTS], finite.  depth: 1..OTHELLO_SEARCH_MAX_DEPTH, else
+ * OTHELLO_E_INVALID.  turn: [n] side to move (OTHELLO_BLACK, anything else = White), or NULL = Black.  Asynchronous on
+ * `stream`, DEVICE pointers, allocates nothing, keeps no global state.  workspace: DEVICE scratch,
+ * >= othello_search_workspace_bytes(); holds the work counter of the persistent grid, which the call resets itself.
+ * n = 0 is a no-op. */
+#define OTHELLO_SEARCH_MAX_DEPTH 12
+int64_t othello_search_workspace_bytes(void);
+int othello_search(const uint64_t *black, const uint64_t *white, const uint8_t *turn, const float *weights,
+                   int32_t depth, float *value, uint8_t *move, uint64_t *nodes, int64_t n, void *workspace,
+                   int64_t workspace_bytes, void *stream);
 
 /* ---- learner sufficient statistics ---------------------------------------------------------- */
 

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libothello_b200.so")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 u64p = ctypes.POINTER(ctypes.c_uint64)
 u8p = ctypes.POINTER(ctypes.c_uint8)
@@ -66,6 +66,8 @@ SIGNATURES = {
                                            ctypes.c_int, vp, i64, vp, vp]),
     "othello_solve_workspace_bytes": (i64, []),
     "othello_solve": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, i64, vp, i64, vp]),
+    "othello_search_workspace_bytes": (i64, []),
+    "othello_search": (ctypes.c_int, [vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, i64, vp]),
     "othello_learn_accumulate": (ctypes.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, vp, vp, vp]),
     "othello_learn_stats": (ctypes.c_int, [vp, vp, vp]),
     "othello_learn_refit": (ctypes.c_int, [vp, i32, vp, vp, vp, vp, vp, vp]),

@@ -17,3 +17,17 @@ static inline int ob_launch_status()
 #define OB_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return (int)e_; } while (0)
 
 static inline unsigned ob_blocks(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
+// The grid of a persistent kernel whose lanes take their work from a counter: as many CTAs as fit on the device at
+// once (a CTA beyond that would only start once the work had run out), fewer for a small n.
+template <typename Kernel>
+static inline int ob_persistent_blocks(Kernel kernel, int threads, int64_t n, unsigned &blocks)
+{
+    int dev = 0, sms = 0, per_sm = 0;
+    OB_CUDA(cudaGetDevice(&dev));
+    OB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    OB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0));
+    const int64_t want = (n + threads - 1) / threads, fit = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
+    blocks = (unsigned)(want < fit ? want : fit);
+    return 0;
+}

@@ -58,13 +58,8 @@ extern "C" int othello_solve(const uint64_t *black, const uint64_t *white, const
     cudaStream_t s = (cudaStream_t)stream;
     unsigned long long *next = (unsigned long long *)workspace;
     OB_CUDA(cudaMemsetAsync(next, 0, sizeof *next, s));
-    // as many CTAs as fit on the device at once: a CTA beyond that would only start once the work had run out
-    int dev = 0, sms = 0, per_sm = 0;
-    OB_CUDA(cudaGetDevice(&dev));
-    OB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    OB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, endgame_kernel, kThreads, 0));
-    const int64_t want = (n + kThreads - 1) / kThreads, fit = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
-    const unsigned blocks = (unsigned)(want < fit ? want : fit);
+    unsigned blocks;
+    if (const int e = ob_persistent_blocks(endgame_kernel, kThreads, n, blocks)) return e;
     endgame_kernel<<<blocks, kThreads, 0, s>>>((const u64 *)black, (const u64 *)white, turn, value, move,
                                                (unsigned long long *)nodes, n, next);
     return ob_launch_status();

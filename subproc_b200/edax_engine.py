@@ -3,7 +3,8 @@
 The reference plays a game by spawning two engines with ``subprocess.Popen(path, shell=True)`` and
 talking to them over pipes (game_runner.py:11-102).  This module is such an engine:
 
-    python -m subproc_b200.edax_engine [--policy random|greedy] [--param FILE] [--name NAME] [--seed S] [--exact N]
+    python -m subproc_b200.edax_engine [--policy random|greedy|search] [--depth D] [--param FILE] [--name NAME]
+                                       [--seed S] [--exact N]
     python -m subproc_b200.edax_engine -h "<64 chars> <turn char>"      # feature dump
 
 Protocol, as read by the reference's regexes:
@@ -17,8 +18,13 @@ Protocol, as read by the reference's regexes:
 the turn character -- what parameter_learn_from_edax_protocol.counts parses (:7-13).  Which colour
 the external engines meant is not pinned by the reference (the engines are not vendored).
 
+``--policy search --depth D`` (D = 1..12, default 4): ``go`` plays the move of a D-ply alpha-beta search on the
+parameter set (ops.search: every leaf scored with the linear evaluation from the engine's side, a pass is a ply; the
+lowest square among the best moves).  Depth 1 is the greedy policy.
+
 ``--exact N`` (default 0 = off): with at most N empty squares left, ``go`` plays the perfect-play move of the exact
-endgame solver (ops.solve; the lowest square among the best moves) instead of the policy's.  N <= 24.
+endgame solver (ops.solve; the lowest square among the best moves) instead of the policy's.  N <= 24.  So
+``--policy search --depth 6 --exact 20`` searches the midgame and plays the endgame perfectly.
 
 Move choice and all rules run through the CUDA kernels (subproc_b200.board / ops).
 """
@@ -29,8 +35,13 @@ import sys
 class Backend(object):
     """rules + policy on the GPU"""
 
-    def __init__(self, policy='random', weights=None, seed=0, device=None, exact_empties=0):
+    def __init__(self, policy='random', weights=None, seed=0, device=None, exact_empties=0, depth=4):
         from . import board
+        if policy == 'search':
+            from . import ops
+            if not 1 <= depth <= ops.SEARCH_MAX_DEPTH:
+                raise ValueError("depth must be in 1..%d" % ops.SEARCH_MAX_DEPTH)
+        self.depth = depth
         if exact_empties:
             from . import ops
             if not 0 < exact_empties <= ops.SOLVE_MAX_EMPTIES:
@@ -69,6 +80,11 @@ class Backend(object):
             x, y = legal[key % len(legal)] if self.policy == 'random' else legal[0]
             return self.b.handstr_from_coord(x, y).upper()
         dev = torch.device("cuda", self.b._ctx_index())
+        w = torch.from_numpy(np.asarray(self.weights, dtype=np.float32).reshape(4, 10)).to(dev)
+        if self.policy == 'search':
+            _, move, _ = ops.search(ops.bits_tensor([own], dev), ops.bits_tensor([opp], dev), w, self.depth)
+            s = int(move[0])
+            return self.b.handstr_from_coord(s & 7, s >> 3).upper()
         n = len(legal)
         sq = torch.tensor([x + 8 * y for x, y in legal], dtype=torch.uint8, device=dev)
         o = ops.bits_tensor([own] * n, dev)
@@ -77,7 +93,6 @@ class Backend(object):
         o2 = o | f | ops.bits_tensor([1 << (x + 8 * y) for x, y in legal], dev)
         p2 = p & ~f
         side = torch.ones(n, dtype=torch.uint8, device=dev)            # evaluate (own', opp') as "Black" = own
-        w = torch.from_numpy(np.asarray(self.weights, dtype=np.float32).reshape(4, 10)).to(dev)
         v = ops.evaluate(o2, p2, side, w).cpu().numpy()
         k = int(np.argmax(v))                                          # first maximum = lowest square
         return self.b.handstr_from_coord(*legal[k]).upper()
@@ -146,7 +161,8 @@ def main(argv=None):
         print(feature_dump(argv[1]))
         return 0
     ap = argparse.ArgumentParser(add_help=False)
-    ap.add_argument("--policy", default="greedy", choices=["random", "greedy"])
+    ap.add_argument("--policy", default="greedy", choices=["random", "greedy", "search"])
+    ap.add_argument("--depth", type=int, default=4, help="plies searched by --policy search (1..12)")
     ap.add_argument("--param", default=None, help="38-byte parameter file (paramgen format)")
     ap.add_argument("--name", default="b200")
     ap.add_argument("--seed", type=int, default=0)
@@ -155,7 +171,7 @@ def main(argv=None):
     from . import parameter, paramgen
     P = parameter.ProgressPositionMovesParameter()
     weights = P.weights_table(paramgen.read_data(args.param) if args.param else None)
-    EdaxFrontEnd(Backend(args.policy, weights, args.seed, exact_empties=args.exact), args.name).serve()
+    EdaxFrontEnd(Backend(args.policy, weights, args.seed, exact_empties=args.exact, depth=args.depth), args.name).serve()
     return 0
 
 

@@ -2,7 +2,8 @@
 
 ``do_match(conf)`` reads the same flat config keys (config.py:4-16 produces ``<section>_<option>``):
 ``proc_a_path`` / ``proc_b_path`` -- here engine specs instead of shell commands: ``random``,
-``greedy`` (default_value() weights) or ``greedy:<38-byte parameter file>`` -- plus
+``greedy`` (default_value() weights), ``greedy:<38-byte parameter file>``, ``search<D>`` (a D-ply alpha-beta search on
+the default_value() weights) or ``search<D>:<parameter file>`` -- plus
 ``proc_n_rand_hands_for_a/b``, ``proc_debug``, ``proc_randomize_black_white`` and the recorder plugin
 ``game_recorder_from`` / ``game_recorder_class``.  Returns what play_a_game returns.
 """
@@ -27,7 +28,12 @@ def engine_from_spec(spec):
         return Engine('greedy', P.weights_table())
     if spec.startswith('greedy:'):
         return Engine('greedy', P.weights_table(paramgen.read_data(spec.split(':', 1)[1])))
-    raise ValueError("unknown engine spec %r (expected random | greedy | greedy:<param file>)" % spec)
+    kind, _, path = spec.partition(':')
+    if kind.startswith('search') and kind[6:].isdigit():
+        table = P.weights_table(paramgen.read_data(path)) if path else P.weights_table()
+        return Engine('search', table, depth=int(kind[6:]))
+    raise ValueError("unknown engine spec %r (expected random | greedy | greedy:<param file> | search<depth> | "
+                     "search<depth>:<param file>)" % spec)
 
 
 def do_match(conf, seed=0, device=None, recorder=None):

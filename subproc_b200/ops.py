@@ -337,6 +337,40 @@ def solve(black, white, turn=None, nodes=False):
     return value, move, cnt
 
 
+SEARCH_MAX_DEPTH = 12                            # OTHELLO_SEARCH_MAX_DEPTH
+_search_ws = {}                                  # (device, stream) -> workspace: the work counter of one call at a time
+
+
+def search(black, white, weights, depth, turn=None, nodes=False):
+    """Depth-limited midgame search on the linear evaluation (othello_search): (value float32 [n], move uint8 [n],
+    nodes int64 [n] or None).
+
+    Every node is scored with ``weights`` (float32 [4][10] on the device) from the side to move at the root (``turn``:
+    uint8 [n], 1 = Black, None = Black to move everywhere); a pass is a ply and uses one level of ``depth``
+    (1..SEARCH_MAX_DEPTH).  value = the minimax value, move = the lowest square reaching it, PASS when the mover must
+    pass, NO_MOVE when the game is over.  depth 1 is the greedy policy.  Positions with overlapping colours get NaN /
+    NO_MOVE.  ``nodes``: also return the positions the search visited, per position (benchmarking)."""
+    if not 1 <= int(depth) <= SEARCH_MAX_DEPTH:
+        raise ValueError("depth must be in 1..%d, got %r" % (SEARCH_MAX_DEPTH, depth))
+    n = black.numel()
+    dev = black.device
+    value = torch.empty(n, dtype=torch.float32, device=dev)
+    move = torch.empty(n, dtype=torch.uint8, device=dev)
+    cnt = torch.empty(n, dtype=torch.int64, device=dev) if nodes else None
+    nbytes = int(_lib.lib().othello_search_workspace_bytes())
+    with torch.cuda.device(dev):
+        stream = _stream(black)
+        ws = _search_ws.get((dev, stream.value))
+        if ws is None:
+            ws = _search_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        _lib.check(_lib.lib().othello_search(
+            _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
+            _req(weights, torch.float32, 40, "weights"), int(depth), _req(value, torch.float32, n, "value"),
+            _req(move, torch.uint8, n, "move"), _opt(cnt, torch.int64, n, "nodes"), n,
+            _req(ws, torch.uint8, nbytes, "workspace"), nbytes, stream), "othello_search")
+    return value, move, cnt
+
+
 def decay_table(t_max, lam=0.90):
     """decay[k] = lam ** k in fp64, evaluated by CPython exactly like `self.l ** turn_left`
     (progress_position_moves_learn.py:24,55)."""
