@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define OTHELLO_ABI_VERSION 5
+#define OTHELLO_ABI_VERSION 6
 
 #define OTHELLO_EMPTY 0
 #define OTHELLO_BLACK 1
@@ -50,6 +50,7 @@ extern "C" {
 /* playout policies: what the two engines behind GameRunner answer to 'go' */
 #define OTHELLO_POLICY_RANDOM 0    /* uniform over puttables(), 'ps' when empty */
 #define OTHELLO_POLICY_GREEDY 1    /* arg-max of the linear evaluation of the successor, ties -> lowest square */
+#define OTHELLO_POLICY_SEARCH 2    /* the move othello_search returns at that colour's depth on that colour's table */
 
 #define OTHELLO_FEATURES   10      /* counts(): discs, mobility, a..h (parameter_progress_position_moves_learn.py:5-17) */
 #define OTHELLO_PHASES      4      /* disc-count shards (0,16),(17,32),(33,48),(49,64) (progress_position_moves_learn.py:112-113) */
@@ -120,7 +121,7 @@ typedef struct {
     int32_t  random_plies;        /* greedy engine answers uniformly at random while ply < random_plies */
     int32_t  n_rand_black;        /* go_for's substitution budget n_rand_hands (game_runner.py:116-119,133-152) */
     int32_t  n_rand_white;
-    const float *weights;         /* DEVICE float[4][10]; required for OTHELLO_POLICY_GREEDY */
+    const float *weights;         /* DEVICE float[4][10]; required for OTHELLO_POLICY_GREEDY / _SEARCH */
     int32_t  t_max;               /* trajectory capacity in plies (120 holds every game from <= 60 empties) */
     int64_t  stride;              /* games per trajectory row (>= n_games); random engine: (t_max + 2) * stride < 2^32 */
     uint64_t *traj_black;         /* [t_max+1][stride] position before ply t (recorder.add, game_runner.py:170,159); NULL = none */
@@ -132,7 +133,7 @@ typedef struct {
     /* proc_black / proc_white may be different engines (GameRunner.__init__, game_runner.py:107-123): */
     int32_t  policy_white;        /* White's engine, or -1 = the same as `policy` (which is then both players') */
     int32_t  games_per_warp;      /* greedy engine: games a warp plays, 8 / 16 / 32; anything else = chosen from n_games */
-    const float *weights_white;   /* DEVICE float[4][10] for White's greedy engine, or NULL = `weights` */
+    const float *weights_white;   /* DEVICE float[4][10] for White's greedy / search engine, or NULL = `weights` */
     /* what GameRunner.play_a_game reports at the end of a game (game_runner.py:194-199) and
      * store_batch_stats sums over a batch (learn_base.py:70-88), accumulated (+=) over the games of
      * this launch: [0] plies played, [1] sum of (n_black - n_white) as two's complement, [2] games Black
@@ -142,6 +143,23 @@ typedef struct {
      * n_white as int8 -- all that store_batch_stats needs of a game (learn_base.py:70-98), and a tenth of
      * the bytes of nplies + the final position when results cross PCIe.  DEVICE uint16[n] or NULL. */
     uint16_t *summary;
+    /* The search engine (OTHELLO_POLICY_SEARCH).  These fields are read only when a side searches.  Such a side answers
+     * 'go' with the move othello_search returns for the position, at its depth, on its table (Black: `weights`; White:
+     * `weights_white`, or `weights` when NULL).  Everything else is the greedy engine's rule, with "arg-max of the
+     * successor's evaluation" replaced by that move:
+     *   - a colour's engine plays uniformly at random while ply < random_plies, and when go_for's substitution fires
+     *     (the same draws, budget min(n_rand, 10) and decrements as the greedy engine);
+     *   - a forced move (one legal move) and a pass are played without a search;
+     *   - the other side may be the random or the greedy engine; a greedy engine is a search engine of depth 1, move
+     *     for move;
+     *   - trajectory rows, nplies, final positions, totals and summary mean what they mean for the other engines, and
+     *     game g depends only on (seed, gid0 + g) and the arguments, not on the batch, the launches, the stream or
+     *     the scheduling.
+     * The games run on a persistent grid: a lane whose game ends takes the next one from a counter in `workspace`. */
+    int32_t  search_depth;        /* Black's search depth, 1..OTHELLO_SEARCH_MAX_DEPTH; also White's when policy_white = -1 */
+    int32_t  search_depth_white;  /* White's search depth, or 0 = search_depth */
+    void    *workspace;           /* DEVICE scratch, >= othello_search_workspace_bytes() (else OTHELLO_E_WORKSPACE); the */
+    int64_t  workspace_bytes;     /* call resets the work counter it holds itself, as othello_search does */
 } othello_playout_args;
 
 /* Device memory kept by the library: the random engine takes the first 8 plies of games that start from the
@@ -150,6 +168,12 @@ typedef struct {
  * 14.6 MB copy) and keeps it until the process exits.  A call on a stream that is being captured into a CUDA graph
  * does not upload it: its kernel plays those plies itself.  Results do not depend on either. */
 int othello_playout(const othello_playout_args *args, void *stream);
+/* Argument checks of othello_playout, all made before anything touches a device (OTHELLO_E_INVALID unless noted):
+ * policy in {RANDOM, GREEDY, SEARCH}, policy_white in {-1, RANDOM, GREEDY, SEARCH}; a greedy or search side has a weight
+ * table; a search side has a depth in 1..OTHELLO_SEARCH_MAX_DEPTH and a workspace of at least
+ * othello_search_workspace_bytes() (OTHELLO_E_WORKSPACE).  n_games = 0 is a no-op.  A call without a search side takes
+ * the random or greedy kernel and reads none of the search fields; the host-buffer front end below has no search
+ * engine. */
 
 /* ---- perft ---------------------------------------------------------------------------------- */
 

@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libothello_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 u64p = ctypes.POINTER(ctypes.c_uint64)
 u8p = ctypes.POINTER(ctypes.c_uint8)
@@ -32,6 +32,7 @@ class PlayoutArgs(ctypes.Structure):
         ("traj_black", vp), ("traj_white", vp), ("traj_move", vp),
         ("nplies", vp), ("final_black", vp), ("final_white", vp),
         ("policy_white", i32), ("games_per_warp", i32), ("weights_white", vp), ("totals", vp), ("summary", vp),
+        ("search_depth", i32), ("search_depth_white", i32), ("workspace", vp), ("workspace_bytes", i64),
     ]
 
 

@@ -346,6 +346,7 @@ int othello_playout_host_async(othello_ctx *c, uint64_t seed, uint64_t gid0, int
         a.nplies = d_np + c0; a.final_black = d_fb + c0; a.final_white = d_fw + c0;
         a.totals = totals ? d_tot : nullptr;
         a.summary = summary ? d_sum + c0 : nullptr;
+        a.search_depth = 0; a.search_depth_white = 0; a.workspace = nullptr; a.workspace_bytes = 0;   // (no search engine)
         rc = othello_playout(&a, st);
         if (rc) return fail(c, rc);
         if (summary) OBH_TRY(cudaMemcpyAsync(summary + c0, d_sum + c0, m * 2, cudaMemcpyDeviceToHost, st));

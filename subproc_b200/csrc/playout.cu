@@ -253,16 +253,29 @@ extern "C" int othello_playout(const othello_playout_args *args, void *stream)
     if (a.n_games == 0) return 0;
     OB_CHECK_ARGS(a.nplies && a.final_black && a.final_white);
     OB_CHECK_ARGS((a.black0 == nullptr) == (a.white0 == nullptr));
-    OB_CHECK_ARGS(a.policy == OTHELLO_POLICY_RANDOM || a.policy == OTHELLO_POLICY_GREEDY);
-    OB_CHECK_ARGS(a.policy_white == -1 || a.policy_white == OTHELLO_POLICY_RANDOM || a.policy_white == OTHELLO_POLICY_GREEDY);
+    auto known = [](int p) { return p == OTHELLO_POLICY_RANDOM || p == OTHELLO_POLICY_GREEDY || p == OTHELLO_POLICY_SEARCH; };
+    OB_CHECK_ARGS(known(a.policy));
+    OB_CHECK_ARGS(a.policy_white == -1 || known(a.policy_white));
     const int policy_white = a.policy_white == -1 ? a.policy : a.policy_white;
-    OB_CHECK_ARGS(a.policy != OTHELLO_POLICY_GREEDY || a.weights != nullptr);
-    OB_CHECK_ARGS(policy_white != OTHELLO_POLICY_GREEDY || a.weights != nullptr || a.weights_white != nullptr);
+    OB_CHECK_ARGS(a.policy == OTHELLO_POLICY_RANDOM || a.weights != nullptr);
+    OB_CHECK_ARGS(policy_white == OTHELLO_POLICY_RANDOM || a.weights != nullptr || a.weights_white != nullptr);
     OB_CHECK_ARGS(a.n_rand_black >= 0 && a.n_rand_white >= 0 && a.random_plies >= 0);
     if (a.traj_black || a.traj_white || a.traj_move)       // (a capacity of 0 plies records only the start position)
         OB_CHECK_ARGS(a.traj_black && a.traj_white && (a.traj_move || a.t_max == 0) && a.t_max >= 0 && a.stride >= a.n_games);
-    const bool greedy = a.policy == OTHELLO_POLICY_GREEDY || policy_white == OTHELLO_POLICY_GREEDY;
     cudaStream_t s = (cudaStream_t)stream;
+    if (a.policy == OTHELLO_POLICY_SEARCH || policy_white == OTHELLO_POLICY_SEARCH) {
+        // the engine of each colour as a search depth: 0 = random, 1 = greedy
+        const int depth_white = a.policy_white == -1 || a.search_depth_white == 0 ? a.search_depth : a.search_depth_white;
+        auto depth_of = [](int policy, int depth) {
+            return policy == OTHELLO_POLICY_SEARCH ? depth : policy == OTHELLO_POLICY_GREEDY ? 1 : 0;
+        };
+        const int depth_b = depth_of(a.policy, a.search_depth), depth_w = depth_of(policy_white, depth_white);
+        OB_CHECK_ARGS(a.policy != OTHELLO_POLICY_SEARCH || (depth_b >= 1 && depth_b <= OTHELLO_SEARCH_MAX_DEPTH));
+        OB_CHECK_ARGS(policy_white != OTHELLO_POLICY_SEARCH || (depth_w >= 1 && depth_w <= OTHELLO_SEARCH_MAX_DEPTH));
+        if (a.workspace == nullptr || a.workspace_bytes < othello_search_workspace_bytes()) return OTHELLO_E_WORKSPACE;
+        return ob_launch_search_playout(a, depth_b, depth_w, s);
+    }
+    const bool greedy = a.policy == OTHELLO_POLICY_GREEDY || policy_white == OTHELLO_POLICY_GREEDY;
     if (greedy) return ob_launch_greedy(a, s);
     return launch(a, s);
 }

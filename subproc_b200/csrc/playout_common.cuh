@@ -72,3 +72,5 @@ __device__ __forceinline__ void add_totals(unsigned long long *totals, bool live
 
 // greedy.cu
 int ob_launch_greedy(const othello_playout_args &a, cudaStream_t s);
+// search_playout.cu: depth_b / depth_w = 0 for a random side, 1 for a greedy one
+int ob_launch_search_playout(const othello_playout_args &a, int depth_b, int depth_w, cudaStream_t s);

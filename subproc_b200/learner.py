@@ -152,6 +152,12 @@ def batch_stats(black_discs, white_discs, black_name='black', white_name='white'
     }
 
 
+def _self_play_policy(depth):
+    """the engine of self-play: greedy, or the midgame search when a depth is given"""
+    from . import ops
+    return ops.POLICY_GREEDY if depth is None else ops.POLICY_SEARCH
+
+
 class ProgressPositionMovesLearn(object):
     """The reference learner's public surface (name / configure / fit_parameter / read_parameters,
     learn_base.py:8-33, progress_position_moves_learn.py:19-35) over on-GPU self-play."""
@@ -238,12 +244,14 @@ class ProgressPositionMovesLearn(object):
         return rows
 
     def self_play_iterations_on_device(self, n_iterations, games_per_rank, seed=0, first_iteration=0, random_plies=10,
-                                       device=None, rank=0, world=1, t_max=120):
+                                       device=None, rank=0, world=1, t_max=120, depth=None):
         """config 5 without host round trips: every iteration is playout -> statistics -> all-reduce ->
         othello_learn_refit -> the next playout reads the new table straight from device memory.  The
         host only enqueues; parameters are copied back once at the end.  Same arithmetic as
         ``self_play_iteration`` on identical statistics (the integer parameters may differ by one where a
-        scaled coefficient sits on an integer boundary: two eigen-solvers, last-ulp differences)."""
+        scaled coefficient sits on an integer boundary: two eigen-solvers, last-ulp differences).
+        ``depth``: None plays greedy games; 1..12 plays search self-play at that depth on the current table (the
+        whole game on the device, so the loop still never waits for the host)."""
         import torch
         from . import ops
         dev = torch.device(device if device is not None else ("cuda:%d" % torch.cuda.current_device()))
@@ -253,8 +261,8 @@ class ProgressPositionMovesLearn(object):
         po = params = fits = None
         for it in range(first_iteration, first_iteration + n_iterations):
             gid0 = (it * world + rank) * games_per_rank
-            po = ops.playout(games_per_rank, seed=seed, gid0=gid0, device=dev, policy=ops.POLICY_GREEDY,
-                             random_plies=random_plies, weights=w, t_max=t_max, out=po)
+            po = ops.playout(games_per_rank, seed=seed, gid0=gid0, device=dev, policy=_self_play_policy(depth),
+                             random_plies=random_plies, weights=w, t_max=t_max, out=po, depth=depth)
             ops.learn_accumulate(po, acc=acc, lam=self.l)
             allreduce_stats(acc)
             # statistics + four regressions + clearing the accumulators: one launch, weights updated in place
@@ -373,16 +381,17 @@ class ProgressPositionMovesLearn(object):
         return po, (mses, scores, params, nsamples)
 
     def self_play_iteration(self, games_per_rank, seed=0, iteration=0, random_plies=10, device=None, rank=0,
-                            world=1, t_max=120):
+                            world=1, t_max=120, depth=None):
         """config 5: greedy self-play with the current weights on this rank's shard of game ids,
-        statistics, all-reduce, refit.  Returns (playout, new parameter rows)."""
+        statistics, all-reduce, refit.  Returns (playout, new parameter rows).  ``depth`` (1..12): search
+        self-play at that depth instead, with the same random plies and game ids (depth 1 plays the greedy games)."""
         import torch
         from . import ops
         dev = torch.device(device if device is not None else ("cuda:%d" % torch.cuda.current_device()))
         w = torch.from_numpy(self.weights_table()).to(dev)
         gid0 = (iteration * world + rank) * games_per_rank
-        po = ops.playout(games_per_rank, seed=seed, gid0=gid0, device=dev, policy=ops.POLICY_GREEDY,
-                         random_plies=random_plies, weights=w, t_max=t_max)
+        po = ops.playout(games_per_rank, seed=seed, gid0=gid0, device=dev, policy=_self_play_policy(depth),
+                         random_plies=random_plies, weights=w, t_max=t_max, depth=depth)
         acc = self.accumulate(po)
         rows = self.learn_from_acc(acc, book_id=(iteration + 1) * world * games_per_rank - 1)
         return po, rows

@@ -18,7 +18,7 @@ EMPTY, BLACK, WHITE = 0, 1, 2                    # board.py:3-7
 PASS = 64                                        # 'ps' / 'PS' (board.py:194)
 START_BLACK = 0x0000000810000000                 # board.py:25
 START_WHITE = 0x0000001008000000                 # board.py:24
-POLICY_RANDOM, POLICY_GREEDY = 0, 1
+POLICY_RANDOM, POLICY_GREEDY, POLICY_SEARCH = 0, 1, 2
 F_MUST_PASS, F_GAME_OVER = 1, 2
 T_MAX_DEFAULT = 120                              # 60 moves + 60 interleaved passes
 
@@ -207,7 +207,8 @@ class Playout:
 
 def playout(n_games, seed=0, gid0=0, device=None, black0=None, white0=None, turn0=None, policy=POLICY_RANDOM,
             random_plies=0, n_rand_black=0, n_rand_white=0, weights=None, t_max=T_MAX_DEFAULT, trajectory=True,
-            out=None, policy_white=None, weights_white=None, totals=None, games_per_warp=0, summary=None):
+            out=None, policy_white=None, weights_white=None, totals=None, games_per_warp=0, summary=None, depth=None,
+            depth_white=None):
     """GameRunner.play_a_game (game_runner.py:165-201) for n_games games in ONE kernel launch.
 
     Game g draws from the counter-based stream (seed, gid0 + g): sharding games over launches or
@@ -215,7 +216,15 @@ def playout(n_games, seed=0, gid0=0, device=None, black0=None, white0=None, turn
     ``totals``: optional int64 [4] device tensor, += (plies, sum of n_black - n_white, Black wins, White
     wins) over the games of this launch -- what play_a_game / store_batch_stats report
     (game_runner.py:194-199, learn_base.py:70-88).
+    ``depth`` / ``depth_white``: search depths (1..SEARCH_MAX_DEPTH) of a POLICY_SEARCH side, Black's and White's;
+    White's defaults to ``depth``.  A search side plays the move ``search`` returns, except on random plies,
+    substituted plies and forced moves, which follow the greedy engine's rules.
     """
+    searching = [p == POLICY_SEARCH for p in (policy, policy if policy_white is None else policy_white)]
+    depth_w = depth if depth_white is None else depth_white
+    for searches, d, side in zip(searching, (depth, depth_w), ("Black", "White")):
+        if searches and not (d is not None and 1 <= int(d) <= SEARCH_MAX_DEPTH):
+            raise ValueError("%s searches: its depth must be in 1..%d, got %r" % (side, SEARCH_MAX_DEPTH, d))
     if device is None:
         device = black0.device if black0 is not None else torch.device("cuda", torch.cuda.current_device())
     device = torch.device(device)
@@ -246,7 +255,14 @@ def playout(n_games, seed=0, gid0=0, device=None, black0=None, white0=None, turn
     a.games_per_warp = games_per_warp                          # greedy engine: 0 = chosen from n_games
     a.summary = _opt(summary, torch.int16, n, "summary")        # per game: plies | (n_black - n_white) << 8
     with torch.cuda.device(device):
-        _lib.check(_lib.lib().othello_playout(ctypes.byref(a), _stream(out.nplies)), "othello_playout")
+        stream = _stream(out.nplies)
+        if any(searching):
+            a.policy_white = policy if policy_white is None else policy_white   # (so White's depth is depth_w)
+            a.search_depth = int(depth) if searching[0] else 0
+            a.search_depth_white = int(depth_w) if searching[1] else 0
+            ws, nbytes = _search_workspace(device, stream)      # the work counter: shared with ``search`` on this stream
+            a.workspace, a.workspace_bytes = ctypes.c_void_p(ws.data_ptr()), nbytes
+        _lib.check(_lib.lib().othello_playout(ctypes.byref(a), stream), "othello_playout")
     return out
 
 
@@ -341,6 +357,16 @@ SEARCH_MAX_DEPTH = 12                            # OTHELLO_SEARCH_MAX_DEPTH
 _search_ws = {}                                  # (device, stream) -> workspace: the work counter of one call at a time
 
 
+def _search_workspace(dev, stream):
+    """the workspace of ``search`` and of search playouts on (dev, stream): calls on one stream run one after the
+    other, so they can share its counter; calls on different streams may overlap, so each stream has its own"""
+    nbytes = int(_lib.lib().othello_search_workspace_bytes())
+    ws = _search_ws.get((dev, stream.value))
+    if ws is None:
+        ws = _search_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    return ws, nbytes
+
+
 def search(black, white, weights, depth, turn=None, nodes=False):
     """Depth-limited midgame search on the linear evaluation (othello_search): (value float32 [n], move uint8 [n],
     nodes int64 [n] or None).
@@ -357,12 +383,9 @@ def search(black, white, weights, depth, turn=None, nodes=False):
     value = torch.empty(n, dtype=torch.float32, device=dev)
     move = torch.empty(n, dtype=torch.uint8, device=dev)
     cnt = torch.empty(n, dtype=torch.int64, device=dev) if nodes else None
-    nbytes = int(_lib.lib().othello_search_workspace_bytes())
     with torch.cuda.device(dev):
         stream = _stream(black)
-        ws = _search_ws.get((dev, stream.value))
-        if ws is None:
-            ws = _search_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        ws, nbytes = _search_workspace(dev, stream)
         _lib.check(_lib.lib().othello_search(
             _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
             _req(weights, torch.float32, 40, "weights"), int(depth), _req(value, torch.float32, n, "value"),
