@@ -250,6 +250,45 @@ int othello_search(const uint64_t *black, const uint64_t *white, const uint8_t *
                    int32_t depth, float *value, uint8_t *move, uint64_t *nodes, int64_t n, void *workspace,
                    int64_t workspace_bytes, void *stream);
 
+/* ---- move values ---------------------------------------------------------------------------- */
+
+/* The value of every move of n positions: rows of OTHELLO_MOVE_SLOTS entries indexed by the move code (squares
+ * 0..63, OTHELLO_PASS).  One lane per (position, move); the rows are written whole, sentinels included.
+ *
+ * othello_search_moves: values float [n][65].
+ *   values[i][s] for a legal square s: the minimax value of the subtree after s, searched to depth - 1 further plies,
+ *                every node scored from the ROOT mover's side as in othello_search.  Each move is searched with a
+ *                full window, so the value is exact and does not depend on pruning, order or scheduling; -0.0 is
+ *                returned as +0.0.  depth = 1: othello_eval of the successor with side = the mover.
+ *   values[i][64] when the mover must pass: the passed position searched to depth - 1, the value othello_search
+ *                returns with move == OTHELLO_PASS.
+ *   NaN everywhere else: illegal squares, the pass column when the mover has a move, every entry of a game-over
+ *   position or of a position with black & white != 0.  So for a position that is not over and has disjoint
+ *   colours, the maximum of the row's finite entries is othello_search's value, bit for bit, and the lowest index
+ *   reaching it its move.  weights, depth (1..OTHELLO_SEARCH_MAX_DEPTH) and turn as for othello_search; workspace
+ *   >= othello_search_workspace_bytes().
+ *
+ * othello_solve_moves: values int32 [n][65].
+ *   values[i][s] for a legal square s: the perfect-play value after s from the mover's side, with othello_solve's
+ *                scoring (empties are not given to the winner) = minus othello_solve of the position after s.
+ *   values[i][64] when the mover must pass: othello_solve's value of the position.
+ *   OTHELLO_SOLVE_REFUSED everywhere else, and in every entry of a position with more than OTHELLO_SOLVE_MAX_EMPTIES
+ *   empties, a game-over position or overlapping colours.  The row's maximum and its lowest arg-max are
+ *   othello_solve's value and move.  workspace >= othello_solve_workspace_bytes().
+ *
+ * Both: nodes: uint64 [n][65] or NULL, the positions each move's search visited (0 where there is no value), a
+ * function of (position, move, depth, weights) alone, whatever the batch.  turn: [n] side to move (OTHELLO_BLACK,
+ * anything else = White), or NULL = Black.  The arguments are checked before anything touches a device:
+ * OTHELLO_E_INVALID for a null pointer, n < 0 or a depth out of range, OTHELLO_E_WORKSPACE for a short workspace;
+ * n = 0 is a no-op.  Asynchronous on `stream`, DEVICE pointers, allocate nothing, keep no global state; the call
+ * resets the work counter it keeps in the workspace itself. */
+#define OTHELLO_MOVE_SLOTS 65
+int othello_search_moves(const uint64_t *black, const uint64_t *white, const uint8_t *turn, const float *weights,
+                         int32_t depth, float *values, uint64_t *nodes, int64_t n, void *workspace,
+                         int64_t workspace_bytes, void *stream);
+int othello_solve_moves(const uint64_t *black, const uint64_t *white, const uint8_t *turn, int32_t *values,
+                        uint64_t *nodes, int64_t n, void *workspace, int64_t workspace_bytes, void *stream);
+
 /* ---- learner sufficient statistics ---------------------------------------------------------- */
 
 /* For every recorded position t of every game and both sides ('O' = Black then 'X' = White,

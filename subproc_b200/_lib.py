@@ -69,6 +69,8 @@ SIGNATURES = {
     "othello_solve": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, i64, vp, i64, vp]),
     "othello_search_workspace_bytes": (i64, []),
     "othello_search": (ctypes.c_int, [vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, i64, vp]),
+    "othello_search_moves": (ctypes.c_int, [vp, vp, vp, vp, i32, vp, vp, i64, vp, i64, vp]),
+    "othello_solve_moves": (ctypes.c_int, [vp, vp, vp, vp, vp, i64, vp, i64, vp]),
     "othello_learn_accumulate": (ctypes.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, vp, vp, vp]),
     "othello_learn_stats": (ctypes.c_int, [vp, vp, vp]),
     "othello_learn_refit": (ctypes.c_int, [vp, i32, vp, vp, vp, vp, vp, vp]),

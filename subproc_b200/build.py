@@ -14,8 +14,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libothello_b200.so")
 SOURCES = ("rules.cu", "playout.cu", "greedy.cu", "perft.cu", "learn.cu", "learn_solve.cu", "value_table.cu", "peak.cu", "host_api.cu",
-           "solve.cu", "search.cu", "search_playout.cu")
-HEADERS = ("bitboard.cuh", "fastboard.cuh", "opening_book.cuh", "endgame.cuh", "midgame.cuh", "playout_common.cuh", "common.cuh", os.path.join("..", "..", "include", "othello_b200.h"))
+           "solve.cu", "search.cu", "search_playout.cu", "move_values.cu")
+HEADERS = ("bitboard.cuh", "fastboard.cuh", "opening_book.cuh", "endgame.cuh", "midgame.cuh", "move_values.cuh", "playout_common.cuh", "common.cuh", os.path.join("..", "..", "include", "othello_b200.h"))
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

@@ -325,6 +325,16 @@ SOLVE_REFUSED = -128                             # OTHELLO_SOLVE_REFUSED
 _solve_ws = {}                                   # (device, stream) -> workspace: the work counter of one call at a time
 
 
+def _solve_workspace(dev, stream):
+    """the workspace of ``solve`` and ``solve_moves`` on (dev, stream): calls on one stream run one after the other, so
+    they can share its counter; calls on different streams may overlap, so each stream has its own"""
+    nbytes = int(_lib.lib().othello_solve_workspace_bytes())
+    ws = _solve_ws.get((dev, stream.value))
+    if ws is None:
+        ws = _solve_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    return ws, nbytes
+
+
 def solve(black, white, turn=None, nodes=False):
     """Exact endgame values (othello_solve): (value int32 [n], move uint8 [n], nodes int64 [n] or None).
 
@@ -338,14 +348,9 @@ def solve(black, white, turn=None, nodes=False):
     value = torch.empty(n, dtype=torch.int32, device=dev)
     move = torch.empty(n, dtype=torch.uint8, device=dev)
     cnt = torch.empty(n, dtype=torch.int64, device=dev) if nodes else None
-    nbytes = int(_lib.lib().othello_solve_workspace_bytes())
     with torch.cuda.device(dev):
         stream = _stream(black)
-        # calls on one stream run one after the other; calls on different streams may overlap, so each stream has
-        # its own counter
-        ws = _solve_ws.get((dev, stream.value))
-        if ws is None:
-            ws = _solve_ws[(dev, stream.value)] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        ws, nbytes = _solve_workspace(dev, stream)
         _lib.check(_lib.lib().othello_solve(
             _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
             _req(value, torch.int32, n, "value"), _req(move, torch.uint8, n, "move"), _opt(cnt, torch.int64, n, "nodes"),
@@ -358,7 +363,7 @@ _search_ws = {}                                  # (device, stream) -> workspace
 
 
 def _search_workspace(dev, stream):
-    """the workspace of ``search`` and of search playouts on (dev, stream): calls on one stream run one after the
+    """the workspace of ``search``, ``search_moves`` and of search playouts on (dev, stream): calls on one stream run one after the
     other, so they can share its counter; calls on different streams may overlap, so each stream has its own"""
     nbytes = int(_lib.lib().othello_search_workspace_bytes())
     ws = _search_ws.get((dev, stream.value))
@@ -392,6 +397,56 @@ def search(black, white, weights, depth, turn=None, nodes=False):
             _req(move, torch.uint8, n, "move"), _opt(cnt, torch.int64, n, "nodes"), n,
             _req(ws, torch.uint8, nbytes, "workspace"), nbytes, stream), "othello_search")
     return value, move, cnt
+
+
+MOVE_SLOTS = 65                                  # OTHELLO_MOVE_SLOTS: a row per position, squares 0..63 and PASS
+
+
+def search_moves(black, white, weights, depth, turn=None, nodes=False):
+    """The search value of every move (othello_search_moves): (values float32 [n][MOVE_SLOTS], nodes int64
+    [n][MOVE_SLOTS] or None).
+
+    values[i][s] = the minimax value of the subtree after square s, searched to ``depth`` - 1 further plies with every
+    node scored from the root mover's side, as ``search`` scores it; values[i][PASS] = the passed position's value when
+    the mover must pass; NaN where there is no such move (and in every entry of a game-over position or of overlapping
+    colours).  The row's maximum and lowest arg-max are ``search``'s value and move.  Only enqueues."""
+    if not 1 <= int(depth) <= SEARCH_MAX_DEPTH:
+        raise ValueError("depth must be in 1..%d, got %r" % (SEARCH_MAX_DEPTH, depth))
+    n = black.numel()
+    dev = black.device
+    values = torch.empty((n, MOVE_SLOTS), dtype=torch.float32, device=dev)
+    cnt = torch.empty((n, MOVE_SLOTS), dtype=torch.int64, device=dev) if nodes else None
+    with torch.cuda.device(dev):
+        stream = _stream(black)
+        ws, nbytes = _search_workspace(dev, stream)
+        _lib.check(_lib.lib().othello_search_moves(
+            _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
+            _req(weights, torch.float32, 40, "weights"), int(depth), _req(values, torch.float32, MOVE_SLOTS * n, "values"),
+            _opt(cnt, torch.int64, MOVE_SLOTS * n, "nodes"), n, _req(ws, torch.uint8, nbytes, "workspace"), nbytes,
+            stream), "othello_search_moves")
+    return values, cnt
+
+
+def solve_moves(black, white, turn=None, nodes=False):
+    """The perfect-play value of every move (othello_solve_moves): (values int32 [n][MOVE_SLOTS], nodes int64
+    [n][MOVE_SLOTS] or None).
+
+    values[i][s] = the value after square s from the mover's side (minus ``solve`` of the child); values[i][PASS] =
+    ``solve``'s value when the mover must pass; SOLVE_REFUSED where there is no such move, and in every entry of a
+    position with more than SOLVE_MAX_EMPTIES empties, a game-over position or overlapping colours.  The row's maximum
+    and lowest arg-max are ``solve``'s value and move.  Only enqueues."""
+    n = black.numel()
+    dev = black.device
+    values = torch.empty((n, MOVE_SLOTS), dtype=torch.int32, device=dev)
+    cnt = torch.empty((n, MOVE_SLOTS), dtype=torch.int64, device=dev) if nodes else None
+    with torch.cuda.device(dev):
+        stream = _stream(black)
+        ws, nbytes = _solve_workspace(dev, stream)
+        _lib.check(_lib.lib().othello_solve_moves(
+            _req(black, torch.int64, n, "black"), _req(white, torch.int64, n, "white"), _opt(turn, torch.uint8, n, "turn"),
+            _req(values, torch.int32, MOVE_SLOTS * n, "values"), _opt(cnt, torch.int64, MOVE_SLOTS * n, "nodes"), n,
+            _req(ws, torch.uint8, nbytes, "workspace"), nbytes, stream), "othello_solve_moves")
+    return values, cnt
 
 
 def decay_table(t_max, lam=0.90):
