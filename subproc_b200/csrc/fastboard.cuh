@@ -214,6 +214,81 @@ OBF_HD void mobility_both(u64 black, u64 white, int &mob_black, int &mob_white)
     mob_white = popc_inter(legal_inter(swapped(q)));
 }
 
+// ---- move generation for four boards at once: the rank-sliced layout ----------------------------
+// Word r of a sliced board holds rank r of four games, game j in byte j; bit x of a byte is still file x.  One rank up
+// or down is the next or previous word, so a flood along a vertical or diagonal direction is one pass over the ranks
+// (one LOP3 per rank for four games, plus a 1-bit shift inside the bytes for a diagonal) instead of a Kogge-Stone
+// flood per game; a rank never straddles a byte, so the horizontal directions are row_up32 as above, the one towards
+// lower files on the bit-reversed word (BREV32 also reverses the order of the games, which does not matter).  The
+// inner mask keeps files a and h out of every diagonal and horizontal run, so no shifted bit or carry crosses into a
+// neighbouring game's byte.  Going in and out of the layout is a 4x4 byte transpose per half-board (8 PRMT).
+
+// byte i of word j <-> byte j of word i (its own inverse)
+OBF_HD void transpose4(u32 &w0, u32 &w1, u32 &w2, u32 &w3)
+{
+    const u32 a = byte_perm(w0, w1, 0x5140u), b = byte_perm(w0, w1, 0x7362u);
+    const u32 c = byte_perm(w2, w3, 0x5140u), d = byte_perm(w2, w3, 0x7362u);
+    w0 = byte_perm(a, c, 0x5410u);
+    w1 = byte_perm(a, c, 0x7632u);
+    w2 = byte_perm(b, d, 0x5410u);
+    w3 = byte_perm(b, d, 0x7632u);
+}
+OBF_HD void to_sliced(const u64 v[4], u32 s[8])
+{
+    for (int j = 0; j < 4; j++) { s[j] = lo32(v[j]); s[4 + j] = hi32(v[j]); }
+    transpose4(s[0], s[1], s[2], s[3]);
+    transpose4(s[4], s[5], s[6], s[7]);
+}
+OBF_HD void from_sliced(u32 s[8], u64 v[4])
+{
+    transpose4(s[0], s[1], s[2], s[3]);
+    transpose4(s[4], s[5], s[6], s[7]);
+    for (int j = 0; j < 4; j++) v[j] = pack(s[j], s[4 + j]);
+}
+
+// Board.puttables (board.py:46-52) of four positions: legal[j] = legal_moves(own[j], opp[j])
+OBF_HD void legal_moves4(const u64 own[4], const u64 opp[4], u64 legal[4])
+{
+    u32 o[8], p[8], m[8], mv[8];
+    to_sliced(own, o);
+    to_sliced(opp, p);
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int r = 0; r < 8; r++) {
+        m[r] = p[r] & kInner32;
+        mv[r] = row_up32(o[r], m[r]) | brev32(row_up32(brev32(o[r]), brev32(m[r])));
+    }
+    // Up the board: u8 / u9 / u7 = the squares of rank r + 1 just beyond a run that starts after an own disc and
+    // reaches rank r, along +8 / +9 (towards file h) / +7 (towards file a); each is also the run carried into rank r + 1.
+    u32 u8 = 0, u9 = 0, u7 = 0;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int r = 1; r < 7; r++) {
+        u8 = p[r] & (o[r - 1] | u8);
+        u9 = (m[r] & ((o[r - 1] << 1) | u9)) << 1;
+        u7 = (m[r] & ((o[r - 1] >> 1) | u7)) >> 1;
+        mv[r + 1] |= u8 | u9 | u7;
+    }
+    // ... and down the board: -8, -9 (towards file a), -7 (towards file h)
+    u32 d8 = 0, d9 = 0, d7 = 0;
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int r = 6; r > 0; r--) {
+        d8 = p[r] & (o[r + 1] | d8);
+        d9 = (m[r] & ((o[r + 1] >> 1) | d9)) >> 1;
+        d7 = (m[r] & ((o[r + 1] << 1) | d7)) << 1;
+        mv[r - 1] |= d8 | d9 | d7;
+    }
+#if defined(__CUDACC__)
+#pragma unroll
+#endif
+    for (int r = 0; r < 8; r++) mv[r] &= ~(o[r] | p[r]);
+    from_sliced(mv, legal);
+}
+
 
 // ---- put(): flips through carry propagation along rays -----------------------------------------
 // ray table: ray[d][s] = squares strictly beyond s in direction d in {+1, +7, +8, +9}, up to the edge; behind the
