@@ -1,6 +1,5 @@
-// bitboard.cuh -- what every kernel shares besides the rules primitives of fastboard.cuh: the
-// square-class masks of the feature code, the phase rows, the counter-based RNG, counts() and the
-// linear evaluation, and the shared-memory ray table that put() needs.
+// bitboard.cuh -- what every kernel shares besides the rules primitives of fastboard.cuh and the linear
+// evaluation of eval.cuh: the counter-based RNG, counts(), and the shared-memory ray table that put() needs.
 //
 // The rules themselves -- the replacement of the reference's list-of-lists ray walks
 // (board.py:124-174: hands_for_direc, is_puttable_at, put) -- are obf::legal_moves / obf::flips_for.
@@ -8,30 +7,9 @@
 #pragma once
 #include <stdint.h>
 #include "fastboard.cuh"
+#include "eval.cuh"
 
 namespace ob {
-
-typedef unsigned long long u64;
-typedef unsigned int u32;
-
-// square-class masks a..h (parameter_progress_position_moves_learn.py:9-16)
-__device__ constexpr u64 kClassMask[8] = {
-    0x8100000000000081ull, 0x4281000000008142ull, 0x0042000000004200ull, 0x2400810000810024ull,
-    0x1800008181000018ull, 0x003C424242423C00ull, 0x0000240000240000ull, 0x0000183C3C180000ull};
-
-// Board.mask_count(side, class k) (board.py:74-81) for the eight classes.  Every class mask is mirror
-// symmetric and its low and high words occupy different bit positions, so the two halves of the board can
-// be merged before counting: one POPC instead of two and no add.
-__device__ __forceinline__ int class_count(u64 bb, int k)
-{
-    const u32 mlo = (u32)kClassMask[k], mhi = (u32)(kClassMask[k] >> 32);
-    return __popc(((u32)bb & mlo) | ((u32)(bb >> 32) & mhi));
-}
-static_assert(((kClassMask[0] >> 32) & kClassMask[0] & 0xffffffffull) == 0 && ((kClassMask[1] >> 32) & kClassMask[1] & 0xffffffffull) == 0 &&
-              ((kClassMask[2] >> 32) & kClassMask[2] & 0xffffffffull) == 0 && ((kClassMask[3] >> 32) & kClassMask[3] & 0xffffffffull) == 0 &&
-              ((kClassMask[4] >> 32) & kClassMask[4] & 0xffffffffull) == 0 && ((kClassMask[5] >> 32) & kClassMask[5] & 0xffffffffull) == 0 &&
-              ((kClassMask[6] >> 32) & kClassMask[6] & 0xffffffffull) == 0 && ((kClassMask[7] >> 32) & kClassMask[7] & 0xffffffffull) == 0,
-              "class masks: low and high words must not share bit positions");
 
 // ---- counter-based RNG (DESIGN.md "RNG"; oracle restatement: orc_rng_*) ----------------------
 __device__ __forceinline__ u32 fmix32(u32 h)
@@ -63,16 +41,7 @@ __device__ __forceinline__ u32 rng_draw_fma(u32 key, u32 ply, u32 stream, u32 on
     return h;
 }
 
-// ---- features / evaluation -------------------------------------------------------------------
-// phase row of a disc count: shards (0,16),(17,32),(33,48),(49,64) inclusive
-// (progress_position_moves_learn.py:75,112-113)
-__device__ __forceinline__ int phase_row(int discs)
-{
-    int r = (discs + 15) >> 4;
-    r -= 1;
-    return r < 0 ? 0 : (r > 3 ? 3 : r);
-}
-
+// ---- features --------------------------------------------------------------------------------
 // counts(a_book, side) (parameter_progress_position_moves_learn.py:5-17) for side = `own`
 __device__ __forceinline__ void features10(u64 own, u64 opp, int f[10])
 {
@@ -80,18 +49,6 @@ __device__ __forceinline__ void features10(u64 own, u64 opp, int f[10])
     f[1] = obf::mobility(own, opp);
 #pragma unroll
     for (int k = 0; k < 8; k++) f[2 + k] = class_count(own, k);
-}
-
-// w[phase] . (mobility, a..h) + w[phase][9]; w = [4][10] floats (shared or global)
-__device__ __forceinline__ float eval_linear(u64 own, u64 opp, const float *__restrict__ w)
-{
-    const int discs = __popcll(own | opp);
-    const float *row = w + 10 * phase_row(discs);
-    float acc = row[9];
-    acc = fmaf(row[0], (float)obf::mobility(own, opp), acc);
-#pragma unroll
-    for (int k = 0; k < 8; k++) acc = fmaf(row[1 + k], (float)class_count(own, k), acc);
-    return acc;
 }
 
 // ray masks for obf::flips_for, [direction][square] so that lanes with different squares spread over

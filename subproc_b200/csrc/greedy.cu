@@ -33,13 +33,6 @@ struct WarpScratch {
     unsigned short item[kMaxItems];           // (White to move << 15) | (game lane << 8) | square
 };
 
-// order-preserving map float -> u32 (larger float <=> larger unsigned); -0.0 is folded into +0.0
-__device__ __forceinline__ unsigned ordered_bits(float v)
-{
-    const unsigned u = __float_as_uint(v + 0.0f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 template <bool SUBST, bool TRAJ>
 #if !defined(OB_GREEDY_CTAS)
 #define OB_GREEDY_CTAS 7
@@ -156,7 +149,7 @@ __global__ void __launch_bounds__(kThreads, OB_GREEDY_CTAS) greedy_kernel(const 
                     const u64 o = ws.own[owner], p = ws.opp[owner];
                     
                     const u64 f = obf::flips_lut<true>((int)sq, o, p, rays, obf::kOpaqueOne);
-                    kbits = ordered_bits(eval_row(o | f | (1ull << sq), p & ~f, w_s + ws.row[owner]));
+                    kbits = ob::ordered_bits(ob::eval_row(o | f | (1ull << sq), p & ~f, w_s + ws.row[owner]));
                     before = ws.best_key[owner];
                 }
                 __syncwarp();

@@ -29,8 +29,8 @@
 // the CPU figure of tools/bench_search.py.
 #pragma once
 #include <math.h>
-#include <string.h>
 #include "endgame.cuh"
+#include "eval.cuh"
 
 namespace obm {
 
@@ -61,52 +61,16 @@ constexpr int kFrames = kMaxDepth - kLowDepth;
 #define OBM_CHECK_FRAME(sp) do { if ((sp) >= kFrames) __builtin_trap(); } while (0)
 #endif
 
-// ---- the evaluation, host+device (ob::eval_linear is device-only) --------------------------------------------------
-// square-class masks a..h (parameter_progress_position_moves_learn.py:9-16), the same as ob::kClassMask
-OBF_HD constexpr u64 class_mask(int k)
-{
-    return k == 0 ? 0x8100000000000081ull : k == 1 ? 0x4281000000008142ull : k == 2 ? 0x0042000000004200ull
-         : k == 3 ? 0x2400810000810024ull : k == 4 ? 0x1800008181000018ull : k == 5 ? 0x003C424242423C00ull
-         : k == 6 ? 0x0000240000240000ull : 0x0000183C3C180000ull;
-}
-
-// phase row of a disc count: shards (0,16),(17,32),(33,48),(49,64) inclusive
-OBF_HD int phase_row(int discs)
-{
-    const int r = ((discs + 15) >> 4) - 1;
-    return r < 0 ? 0 : (r > 3 ? 3 : r);
-}
-
-// w[phase] . (mobility, a..h) + w[phase][9] of colour P: ob::eval_linear's operations in its order
+// score(P, O) of colour P: the linear evaluation of eval.cuh, the value othello_eval returns
 OBF_HD float score(u64 P, u64 O, const float *w)
 {
-    const float *row = w + 10 * phase_row(obf::popc64(P | O));
-    float acc = row[9];
-    acc = fmaf(row[0], (float)obf::mobility(P, O), acc);
-#if defined(__CUDA_ARCH__)
-#pragma unroll
-#endif
-    for (int k = 0; k < 8; k++) acc = fmaf(row[1 + k], (float)obf::popc64(P & class_mask(k)), acc);
-    return acc;
+    return ob::eval_linear(P, O, w);
 }
 
 // the leaf value of a node, from its mover's (`own`) side: sgn = +1 when `own` is the root mover
 OBF_HD float leaf(u64 own, u64 opp, int sgn, const float *w)
 {
     return sgn > 0 ? score(own, opp, w) : -score(opp, own, w);
-}
-
-// order-preserving map float -> u32 (larger float <=> larger unsigned); -0.0 is folded into +0.0
-OBF_HD u32 ordered_bits(float v)
-{
-    v += 0.0f;
-#if defined(__CUDA_ARCH__)
-    const u32 u = __float_as_uint(v);
-#else
-    u32 u;
-    memcpy(&u, &v, sizeof u);
-#endif
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
 // ---- the last plies: register-resident, ascending squares -----------------------------------------------------------
@@ -173,7 +137,7 @@ OBF_HD int order_moves(unsigned char *order, u64 own, u64 opp, u64 legal, int sg
         const int sq = obe::ctz64(rem);
         const u64 f = obf::flips_for(sq, own, opp, own_r, opp_r, rays);
         const float v = leaf(own | f | (1ull << sq), opp & ~f, sgn, w);
-        const u32 k = (~ordered_bits(v) & ~63u) | (u32)sq;
+        const u32 k = (~ob::ordered_bits(v) & ~63u) | (u32)sq;
         int j = n++;
         for (; j > 0 && key[j - 1] > k; j--) key[j] = key[j - 1];
         key[j] = k;

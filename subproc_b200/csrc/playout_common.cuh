@@ -13,29 +13,6 @@ constexpr int kThreads = 128;
 using ob::Rays;
 using ob::fill_rays;
 
-// w[phase] . (mobility, a..h) + w[phase][9] with the tuned move generator
-__device__ __forceinline__ float eval_fast(u64 own, u64 opp, const float *__restrict__ w)
-{
-    const int discs = __popcll(own | opp);
-    const float *row = w + 10 * ob::phase_row(discs);
-    float acc = row[9];
-    acc = fmaf(row[0], (float)obf::mobility(own, opp), acc);
-#pragma unroll
-    for (int k = 0; k < 8; k++) acc = fmaf(row[1 + k], (float)ob::class_count(own, k), acc);
-    return acc;
-}
-
-// the same with the phase row already known (row = w + 10 * phase_row(discs)): the children of one position all
-// have its disc count + 1
-__device__ __forceinline__ float eval_row(u64 own, u64 opp, const float *__restrict__ row)
-{
-    float acc = row[9];
-    acc = fmaf(row[0], (float)obf::mobility(own, opp), acc);
-#pragma unroll
-    for (int k = 0; k < 8; k++) acc = fmaf(row[1 + k], (float)ob::class_count(own, k), acc);
-    return acc;
-}
-
 // go_for's substitution test (game_runner.py:134-135): with budget `rest` left, play a random move
 // with probability 1/rest (stream 0 of the counter-based RNG)
 __device__ __forceinline__ bool substitute_now(u32 key, int t, int rest)

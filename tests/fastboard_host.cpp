@@ -1,21 +1,7 @@
 // tests/fastboard_host.cpp -- TEST SCAFFOLDING: compiles subproc_b200/csrc/fastboard.cuh for the
 // host so the exact source the kernels use can be compared with the oracle without a GPU.
 #include "../subproc_b200/csrc/fastboard.cuh"
-
-static unsigned long long g_rays[obf::kRayTable64];
-static bool g_init = false;
-struct Rays {
-    unsigned long long operator()(int d, int s) const { return g_rays[d * 64 + s]; }
-    unsigned long long word(unsigned i) const { return g_rays[i]; }
-    unsigned byte(unsigned i) const { return ((const unsigned char *)g_rays)[i]; }     // (little-endian host)
-};
-
-static void init()
-{
-    if (g_init) return;
-    for (int i = 0; i < obf::kRayTable64; i++) g_rays[i] = obf::make_table_word(i);
-    g_init = true;
-}
+#include "host_rays.h"
 
 extern "C" void fb_legal(const unsigned long long *own, const unsigned long long *opp, unsigned long long *out, long n)
 {
@@ -25,7 +11,6 @@ extern "C" void fb_legal(const unsigned long long *own, const unsigned long long
 extern "C" void fb_flips(const unsigned long long *own, const unsigned long long *opp, const unsigned char *sq,
                          unsigned long long *out, long n)
 {
-    init();
     for (long i = 0; i < n; i++) {
         const unsigned long long x = 1ull << sq[i];
         out[i] = ((own[i] | opp[i]) & x) ? 0ull
@@ -37,7 +22,6 @@ extern "C" void fb_flips(const unsigned long long *own, const unsigned long long
 extern "C" void fb_flips_rowlut(const unsigned long long *own, const unsigned long long *opp, const unsigned char *sq,
                                 unsigned long long *out, long n)
 {
-    init();
     for (long i = 0; i < n; i++) {
         const unsigned long long x = 1ull << sq[i];
         out[i] = ((own[i] | opp[i]) & x) ? 0ull
@@ -58,7 +42,6 @@ extern "C" void fb_mobility(const unsigned long long *own, const unsigned long l
 extern "C" void fb_child_mobility(const unsigned long long *own, const unsigned long long *opp, const unsigned char *sq,
                                   int *out, long n)
 {
-    init();
     for (long i = 0; i < n; i++) {
         const unsigned long long x = 1ull << sq[i];
         const unsigned long long f = ((own[i] | opp[i]) & x) ? 0ull
@@ -71,7 +54,6 @@ extern "C" void fb_child_mobility(const unsigned long long *own, const unsigned 
 extern "C" void fb_flips_lut(const unsigned long long *own, const unsigned long long *opp, const unsigned char *sq,
                              unsigned long long *out, long n)
 {
-    init();
     for (long i = 0; i < n; i++) {
         const unsigned long long x = 1ull << sq[i];
         out[i] = ((own[i] | opp[i]) & x) ? 0ull : obf::flips_lut(sq[i], own[i], opp[i], Rays(), 1u);
@@ -82,7 +64,6 @@ extern "C" void fb_flips_lut(const unsigned long long *own, const unsigned long 
 extern "C" void fb_flips_lut_line(const unsigned long long *own, const unsigned long long *opp, const unsigned char *sq,
                              unsigned long long *out, long n)
 {
-    init();
     for (long i = 0; i < n; i++) {
         const unsigned long long x = 1ull << sq[i];
         out[i] = ((own[i] | opp[i]) & x) ? 0ull : obf::flips_lut<true>(sq[i], own[i], opp[i], Rays(), 1u);
@@ -92,6 +73,5 @@ extern "C" void fb_flips_lut_line(const unsigned long long *own, const unsigned 
 // byte [value][k] of the k-th-set-bit table the playout kernel reads from shared memory
 extern "C" int fb_kth_table(int value, int k)
 {
-    init();
     return (int)Rays().byte(obf::kKthBit64 * 8 + value * 8 + k);
 }

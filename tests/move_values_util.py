@@ -1,36 +1,22 @@
 """Helpers of the move-value tests: the host build of the rows the kernels write (tests/move_values_host.cpp ->
-csrc/move_values.cuh), built once per process into a temporary directory, run over threads (ctypes releases the
-GIL); and the row reductions the tests compare with othello_search / othello_solve."""
+csrc/move_values.cuh), built once per process (tests/host_build.py), run over threads (ctypes releases the GIL); and
+the row reductions the tests compare with othello_search / othello_solve."""
 import ctypes
 import os
-import subprocess
-import tempfile
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
+import host_build
 import search_util as xu
+from solve_util import _inputs, _p
 
-HERE = os.path.dirname(os.path.abspath(__file__))
 SLOTS = 65
 REFUSED = -128
 
-_lib = []
-
 
 def host_lib():
-    if not _lib:
-        out = os.path.join(tempfile.mkdtemp(prefix="move_values_"), "move_values_host.so")
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                               os.path.join(HERE, "move_values_host.cpp"), "-o", out])
-        L = ctypes.CDLL(out)
-        L.mv_init()
-        _lib.append(L)
-    return _lib[0]
-
-
-def _p(a):
-    return a.ctypes.data_as(ctypes.c_void_p)
+    return host_build.load("move_values_host.cpp")
 
 
 def _split(n, run, threads=None):
@@ -42,7 +28,7 @@ def _split(n, run, threads=None):
 
 def host_search_moves(black, white, turn, weights, depth):
     """(values float32 [n][65], nodes uint64 [n][65]) of the host build"""
-    b, w, t = xu._inputs(black, white, turn)
+    b, w, t = _inputs(black, white, turn)
     n = b.size
     values, nodes = np.zeros((n, SLOTS), np.float32), np.zeros((n, SLOTS), np.uint64)
     wf = xu.weights40(weights)
@@ -54,7 +40,7 @@ def host_search_moves(black, white, turn, weights, depth):
 
 def host_solve_moves(black, white, turn):
     """(values int32 [n][65], nodes uint64 [n][65]) of the host build"""
-    b, w, t = xu._inputs(black, white, turn)
+    b, w, t = _inputs(black, white, turn)
     n = b.size
     values, nodes = np.zeros((n, SLOTS), np.int32), np.zeros((n, SLOTS), np.uint64)
     L = host_lib()

@@ -3,14 +3,7 @@
 // Build it with -std=c++17 (not gnu++17): g++ then contracts no float expression, and only the explicit fmaf fuses,
 // as on the device.
 #include "../subproc_b200/csrc/midgame.cuh"
-
-static unsigned long long g_rays[obf::kRayTable64];
-static bool g_init = false;
-struct Rays {
-    unsigned long long operator()(int d, int s) const { return g_rays[d * 64 + s]; }
-    unsigned long long word(unsigned i) const { return g_rays[i]; }
-    unsigned byte(unsigned i) const { return ((const unsigned char *)g_rays)[i]; }     // (little-endian host)
-};
+#include "host_rays.h"
 
 // black, white, turn (1 = Black, anything else = White; NULL = Black), weights [4][10], depth -> value, move, nodes
 // (NULL = not wanted)
@@ -18,10 +11,6 @@ extern "C" void mg_search(const unsigned long long *black, const unsigned long l
                           const float *weights, int depth, float *value, unsigned char *move, unsigned long long *nodes,
                           long n)
 {
-    if (!g_init) {
-        for (int i = 0; i < obf::kRayTable64; i++) g_rays[i] = obf::make_table_word(i);
-        g_init = true;
-    }
     obm::Frame st[obm::kFrames];
     for (long i = 0; i < n; i++) {
         const bool black_moves = turn ? turn[i] == 1 : true;

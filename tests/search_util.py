@@ -2,48 +2,31 @@
 alpha-beta on the oracle's mailbox rules and fp64 evaluation), the host build of the search the kernel runs
 (tests/search_host.cpp -> csrc/midgame.cuh), weight tables and sampled positions.
 
-Both shared objects are built once per process into a temporary directory."""
+Both shared objects are built once per process (tests/host_build.py)."""
 import ctypes
 import os
-import subprocess
-import tempfile
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
+import host_build
 import solve_util as su
+from solve_util import _inputs, _p
 
-HERE = os.path.dirname(os.path.abspath(__file__))
 BLACK, WHITE, PASS, NO_MOVE = su.BLACK, su.WHITE, su.PASS, su.NO_MOVE
 MAX_DEPTH = 12
 
-_libs = {}
-
-
-def _build(name, cmd):
-    if name not in _libs:
-        out = os.path.join(tempfile.mkdtemp(prefix="search_"), name + ".so")
-        subprocess.check_call(cmd + ["-o", out])
-        _libs[name] = ctypes.CDLL(out)
-    return _libs[name]
-
 
 def oracle_lib():
-    return _build("search_oracle", ["gcc", "-O2", "-std=c99", "-shared", "-fPIC", os.path.join(HERE, "search_oracle.c"),
-                                    "-lm"])
+    return host_build.load("search_oracle.c")
 
 
 def host_lib():
-    """the host build of csrc/midgame.cuh; -std=c++17 so that g++ contracts no float expression"""
-    L = _build("search_host", ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                               os.path.join(HERE, "search_host.cpp")])
+    """the host build of csrc/midgame.cuh"""
+    L = host_build.load("search_host.cpp")
     L.mg_score.restype = ctypes.c_float
     L.mg_score.argtypes = [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p]
     return L
-
-
-def _p(a):
-    return a.ctypes.data_as(ctypes.c_void_p)
 
 
 def weights40(w):
@@ -63,13 +46,6 @@ def int_weights(seed):
 def float_weights(seed):
     """a random three-decimal table with intercepts: scores are not integers, sums round"""
     return weights40(np.round(np.random.RandomState(seed).uniform(-20, 20, size=(4, 10)), 3))
-
-
-def _inputs(black, white, turn):
-    b = np.ascontiguousarray(np.asarray(black, dtype=np.uint64).reshape(-1))
-    w = np.ascontiguousarray(np.asarray(white, dtype=np.uint64).reshape(-1))
-    t = np.full(b.size, BLACK, np.uint8) if turn is None else np.ascontiguousarray(np.asarray(turn, dtype=np.uint8).reshape(-1))
-    return b, w, t
 
 
 def oracle_search(black, white, turn, weights, depth, pruned=False, threads=None):

@@ -2,40 +2,28 @@
 mailbox rules), the host build of the search the kernel runs (tests/solve_host.cpp -> csrc/endgame.cuh), and
 positions with a given number of empty squares from seeded oracle playouts.
 
-Both shared objects are built once per process into a temporary directory."""
+Both shared objects are built once per process (tests/host_build.py)."""
 import ctypes
 import os
-import subprocess
-import tempfile
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
-HERE = os.path.dirname(os.path.abspath(__file__))
+import host_build
+
 BLACK, WHITE = 1, 2
 PASS, NO_MOVE, REFUSED = 64, 255, -128
 
-_libs = {}
 _solved = {}                                     # (black, white, turn, pruned) -> (value, move) of the reference
 
 
-def _build(name, cmd):
-    if name not in _libs:
-        out = os.path.join(tempfile.mkdtemp(prefix="solve_"), name + ".so")
-        subprocess.check_call(cmd + ["-o", out])
-        _libs[name] = ctypes.CDLL(out)
-    return _libs[name]
-
-
 def oracle_lib():
-    return _build("solve_oracle", ["gcc", "-O2", "-std=c99", "-shared", "-fPIC", os.path.join(HERE, "solve_oracle.c"), "-lm"])
+    return host_build.load("solve_oracle.c")
 
 
 def host_lib(defines=()):
     """the host build of csrc/endgame.cuh; defines (e.g. "OBE_MAX_EMPTIES=12") build a variant of the search"""
-    return _build("solve_host" + "".join("_" + d.replace("=", "") for d in defines),
-                  ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++"] + ["-D" + d for d in defines] +
-                  [os.path.join(HERE, "solve_host.cpp")])
+    return host_build.load("solve_host.cpp", defines)
 
 
 def _p(a):

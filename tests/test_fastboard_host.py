@@ -2,23 +2,16 @@
 rotation, carry-propagation rows and rays) compiled for the HOST and compared with the oracle.
 Same source as the kernels, so algorithmic slips are caught on the CPU box."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-SO = os.path.join(HERE, "fastboard_host.so")
+import host_build
 
 
 @pytest.fixture(scope="module")
 def fb():
-    src = os.path.join(HERE, "fastboard_host.cpp")
-    hdr = os.path.join(HERE, "..", "subproc_b200", "csrc", "fastboard.cuh")
-    if not os.path.isfile(SO) or os.path.getmtime(SO) < max(os.path.getmtime(src), os.path.getmtime(hdr)):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++", src, "-o", SO])
-    return ctypes.CDLL(SO)
+    return host_build.load("fastboard_host.cpp")
 
 
 def P(a):

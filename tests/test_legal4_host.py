@@ -1,21 +1,16 @@
 """The rank-sliced move generator of four boards at once (obf::legal_moves4 in csrc/fastboard.cuh, what the random
 playout kernel runs) compiled for the HOST and compared with the oracle and with the one-board generator."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
+import host_build
 
 
 @pytest.fixture(scope="module")
-def fb(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("legal4") / "legal4_host.so")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                           os.path.join(HERE, "legal4_host.cpp"), "-o", so])
-    return ctypes.CDLL(so)
+def fb():
+    return host_build.load("legal4_host.cpp")
 
 
 def P(a):

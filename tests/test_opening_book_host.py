@@ -1,13 +1,11 @@
 """The opening book of the random playout kernel (csrc/opening_book.cuh) compiled for the HOST and compared with the
 oracle: the tree the kernel walks for the first plies of every game from the standard opening."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
+import host_build
 
 NODE = np.dtype([("black", "<u8"), ("white", "<u8"), ("first", "<u4"), ("info", "<u4"), ("pad", "<u4", (2,))])
 # perft from the standard opening (BASELINE.md): move paths after 0..8 plies
@@ -15,11 +13,8 @@ PERFT = [1, 4, 12, 56, 244, 1396, 8200, 55092, 390216]
 
 
 @pytest.fixture(scope="module")
-def book(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("book") / "opening_book_host.so")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                           os.path.join(HERE, "opening_book_host.cpp"), "-o", so])
-    L = ctypes.CDLL(so)
+def book():
+    L = host_build.load("opening_book_host.cpp")
     L.ob_book_build.restype = ctypes.c_long
     L.ob_book_build.argtypes = [ctypes.c_int]
     L.ob_book_copy.argtypes = [ctypes.c_void_p]

@@ -6,7 +6,7 @@ Positions with exactly E empty squares come from seeded random playouts on the G
 of each game that has E empties, in game order, so the sample is fixed by the seed and two builds search the same set.
 Per (table, E, depth): one JSON line with the positions, kernel time (CUDA events around ops.search, after one warm-up
 call of the same shape), positions/s, nodes/s, mean and max nodes per position, and the host build of
-csrc/midgame.cuh (tests/search_host.cpp, compiled into a temporary directory) on the first --cpu positions on one
+csrc/midgame.cuh (tests/search_host.cpp, compiled by tests/host_build.py) on the first --cpu positions on one
 core, whose results must equal the kernel's bit for bit.  Two tables: default_value() and a learnt-looking integer
 table.  GPU name, power limit and SM clocks are read with nvidia-smi (queries only) in the same run.
 """
@@ -14,9 +14,7 @@ import argparse
 import ctypes
 import json
 import os
-import subprocess
 import sys
-import tempfile
 import time
 
 import numpy as np
@@ -25,8 +23,10 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 from subproc_b200 import ops  # noqa: E402
 from bench_solve import gpu_info, positions  # noqa: E402
+import host_build  # noqa: E402
 
 # default_value() (parameter_progress_position_moves_learn.py:30-36) and a table shaped like a learnt one: corners and
 # mobility high, X- and C-squares negative, intercepts non-zero
@@ -36,13 +36,6 @@ TABLES = {
     "learnt": [[12, 61, -38, -17, 9, 4, -2, 3, 1, -6], [15, 57, -29, -12, 6, 3, -1, 2, 2, -4],
                [11, 48, -18, -8, 5, 4, 1, 3, 2, 3], [4, 39, -6, -3, 4, 5, 3, 4, 3, 9]],
 }
-
-
-def host_searcher():
-    out = os.path.join(tempfile.mkdtemp(prefix="bench_search_"), "search_host.so")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                           os.path.join(ROOT, "tests", "search_host.cpp"), "-o", out])
-    return ctypes.CDLL(out)
 
 
 def host_search(L, b, w, t, weights, depth):
@@ -67,7 +60,7 @@ def main():
     assert torch.cuda.is_available(), "bench_search needs a CUDA device"
     dev = torch.device("cuda:0")
     info = gpu_info()
-    L = host_searcher()
+    L = host_build.load("search_host.cpp")
     for name, rows in TABLES.items():
         wh = np.ascontiguousarray(np.asarray(rows, np.float32))
         wd = torch.from_numpy(wh).to(dev)

@@ -5,8 +5,8 @@
 Positions with exactly E empty squares come from seeded random playouts on the GPU (ops.playout): the first position
 of each game that has E empties, in game order, so the sample is fixed by the seed and two builds solve the same set.
 Per E: one JSON line with the positions, kernel time (CUDA events around ops.solve, after one warm-up call), positions/s,
-nodes/s, mean and max nodes per position, and the host build of csrc/endgame.cuh (tests/solve_host.cpp, compiled into a
-temporary directory) on the first --cpu positions on one core.  A call at E empties lasts as long as its slowest
+nodes/s, mean and max nodes per position, and the host build of csrc/endgame.cuh (tests/solve_host.cpp, compiled by
+tests/host_build.py) on the first --cpu positions on one core.  A call at E empties lasts as long as its slowest
 position (one lane solves one position), so the counts shrink with E.  GPU name, power limit and SM clocks are read
 with nvidia-smi (queries only) in the same run.
 """
@@ -16,7 +16,6 @@ import json
 import os
 import subprocess
 import sys
-import tempfile
 import time
 
 import numpy as np
@@ -24,7 +23,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 from subproc_b200 import ops  # noqa: E402
+import host_build  # noqa: E402
 
 
 def gpu_info():
@@ -60,13 +61,6 @@ def positions(empties, n_games, seed, dev):
     return b, w, turn
 
 
-def host_solver():
-    out = os.path.join(tempfile.mkdtemp(prefix="bench_solve_"), "solve_host.so")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++",
-                           os.path.join(ROOT, "tests", "solve_host.cpp"), "-o", out])
-    return ctypes.CDLL(out)
-
-
 def host_solve(L, b, w, t):
     n = b.size
     p = lambda a: a.ctypes.data_as(ctypes.c_void_p)
@@ -98,7 +92,7 @@ def main():
     assert torch.cuda.is_available(), "bench_solve needs a CUDA device"
     dev = torch.device("cuda:0")
     info = gpu_info()
-    L = host_solver()
+    L = host_build.load("solve_host.cpp")
     warm = True
     for e in [int(x) for x in args.empties.split(",")]:
         b, w, t = positions(e, args.games, args.seed + e, dev)
